@@ -2,7 +2,7 @@
 """Benchmark of the projected-LMC hot path (contract: see the repo brief / DESIGN.md section 6).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c1|c2|c3|c4|c5]
-                    [--scaling weak|strong]
+                    [--scaling weak|strong] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Default workload (BASELINE.json configs[1], "C2"): synthetic SARCOS-shaped projected LMC, n = 44,484 points, d = 21,
@@ -13,6 +13,12 @@ parameter, AdamW step, learning-rate scheduler step.  `value` counts 4-latent SA
 second (N per step at N GPUs).  --scaling strong keeps the NAMED model fixed and splits its latents over the ranks
 (C2: 4 latents -> at most 4 GPUs; C4: 32 latents; C5: 8 latents).  c3 is the prediction config (metric: predictive
 mean/variance points per second; test points are sharded over the ranks, every rank holds all factors).
+
+--dump-outputs DIR writes, after the timed steps, what the timed path handed its caller in its last step as
+DIR/<name>.npy (float32 or float64, at most 64 MB in all; larger outputs as a fixed, seeded sample of their rows).
+Training workloads: `loss`, `grad.<parameter>` and `param.<parameter>` (after the optimiser step), and, with the
+prediction section on, `predict.mean` / `predict.variance`; c3: `predict.mean` / `predict.variance`.  Inputs depend
+only on the arguments, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -49,12 +55,20 @@ WORKLOADS = {
 CPU_FIT_NS = (1000, 2000, 4000)          # in-line cpu_baseline of the default run (~10 s of host work)
 REFERENCE_FIT_NS = (2000, 4000, 8000)    # --impl reference (~1-2 min of host work)
 LIBRARY_N = 8192                         # torch -> cuSOLVER restatement on the same GPU
+DUMP_BYTES = 64 << 20                    # cap of everything --dump-outputs writes
+
+
+def positive_int(text):
+    v = int(text)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {v}")
+    return v
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=0, help="timed steps (default: per workload)")
+    ap.add_argument("--steps", type=positive_int, default=None, help="timed steps (default: per workload)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c2", choices=list(WORKLOADS))
@@ -68,7 +82,40 @@ def parse():
     ap.add_argument("--test-points", type=int, default=0)
     ap.add_argument("--dtype", default="f64", choices=["f64", "f32"],
                     help="f32: float32 model -> fp32-grade arithmetic (32-bit operands on the INT8 path, FP64 storage)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy")
     return ap.parse_args()
+
+
+def sample_rows(n_rows, row_bytes, budget, seed=0):
+    """Sorted row indices of a fixed, seeded sample of an [n_rows, ...] output that fits `budget` bytes
+    (None: every row fits)."""
+    k = min(n_rows, max(0, int(budget // max(row_bytes, 1))))
+    if k == n_rows:
+        return None
+    g = torch.Generator().manual_seed(seed)
+    return torch.randperm(n_rows, generator=g)[:k].sort().values
+
+
+def host_outputs(named):
+    """name -> detached host copy (float32 stays float32, everything else becomes float64)."""
+    out = {}
+    for name, t in named.items():
+        t = t.detach().cpu()
+        out[name] = t.clone() if t.dtype in (torch.float32, torch.float64) else t.to(torch.float64)
+    return out
+
+
+def write_outputs(path, arrays):
+    """Writes name -> host tensor as path/<name>.npy; refuses to write more than DUMP_BYTES in all."""
+    import numpy as np
+
+    total = sum(a.numel() * a.element_size() for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_BYTES}-byte cap")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a.numpy())
 
 
 def model_shape(cfg, world, scaling):
@@ -528,6 +575,8 @@ def main():
     cfg = WORKLOADS[args.workload]
     torch.set_default_dtype(torch.float64)
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the outputs of the GPU path (--impl ours)")
         run_reference(args, cfg)
         return
 
@@ -663,6 +712,17 @@ def run_train_workload(args, cfg, world, rank, dev):
     ms_per_step = float(ms.item())
     models_per_step = 1 if args.scaling == "strong" else world
     value = models_per_step / (ms_per_step * 1e-3)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        # the last timed step's loss and gradients, and the parameters its optimiser step left (the e2e steps below
+        # move them on)
+        named = {"loss": loss}
+        for name, prm in model.named_parameters():
+            if prm.requires_grad:
+                named["param." + name] = prm
+                if prm.grad is not None:
+                    named["grad." + name] = prm.grad
+        dump = host_outputs(named)
 
     # ---- end to end: host buffers in, loss out, every step -------------------------
     e2e = None
@@ -715,6 +775,11 @@ def run_train_workload(args, cfg, world, rank, dev):
         if world > 1:
             dist.all_reduce(ms3, op=dist.ReduceOp.MAX)
         pred_s = float(ms3.item()) * 1e-3
+        if dump is not None:
+            out = host_outputs({"predict.mean": pred.mean, "predict.variance": pred.variance})
+            used = sum(a.numel() * a.element_size() for a in dump.values())
+            rows = sample_rows(n_test, sum(a[0].numel() * a.element_size() for a in out.values()), DUMP_BYTES - used)
+            dump.update(out if rows is None else {k: a[rows] for k, a in out.items()})
         predict = {"points_per_sec": n_test / pred_s, "n_test": n_test, "seconds": pred_s,
                    "factorisation_seconds_excluded": fact_s, "checksum": chk,
                    "variance_path": "explicit inverse of the factor (once, in the excluded call) + triangular multiply",
@@ -773,6 +838,8 @@ def run_train_workload(args, cfg, world, rank, dev):
                     "sample": baseline_sample_text(cfg, cfg["p"], cfg["q"], samples, e, n, t, cores),
                     "fitted_exponent": e, "samples_n_seconds": samples, "extrapolated": e is not None,
                 }
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(line), flush=True)
 
 
@@ -825,8 +892,16 @@ def run_predict_workload(args, cfg, world, rank, dev):
         i8_peak = i8_peak_tops()
         peak = dmma_peak_tflops()
         eng = model._engine
+        keep = None
+        if args.dump_outputs:
+            # this rank's rows of a fixed sample of the [n_test, p] outputs, per chunk, gathered in the last timed step
+            rows = sample_rows(n_test, 2 * p * 8, DUMP_BYTES)
+            rows = torch.arange(n_test) if rows is None else rows
+            rows = rows[(rows >= lo) & (rows < hi)] - lo
+            keep = {"rows": {s0: (rows[(rows >= s0) & (rows < s0 + chunk)] - s0).to(dev)
+                             for s0 in range(0, hi - lo, chunk)}, "mean": [], "variance": []}
 
-        def run(from_host):
+        def run(from_host, keep=None):
             chk = torch.zeros((), dtype=torch.float64, device=dev)
             for s0 in range(0, hi - lo, chunk):
                 s1 = min(hi - lo, s0 + chunk)
@@ -835,6 +910,9 @@ def run_predict_workload(args, cfg, world, rank, dev):
                 if from_host:
                     mean_h[s0:s1].copy_(pred.mean, non_blocking=True)
                     var_h[s0:s1].copy_(pred.variance, non_blocking=True)
+                if keep is not None:
+                    keep["mean"].append(pred.mean[keep["rows"][s0]])
+                    keep["variance"].append(pred.variance[keep["rows"][s0]])
                 chk = chk + pred.mean.sum() + pred.variance.sum()
             return chk
 
@@ -842,8 +920,8 @@ def run_predict_workload(args, cfg, world, rank, dev):
         t_wall0 = time.time()
         ops.stats_reset()
         e0.record()
-        for _ in range(steps):
-            chk = run(False)
+        for it in range(steps):
+            chk = run(False, keep if it == steps - 1 else None)
         e1.record()
         barrier()
         clocks = sampler.stop(t_wall0, time.time())
@@ -866,6 +944,13 @@ def run_predict_workload(args, cfg, world, rank, dev):
                 dist.all_reduce(ms2, op=dist.ReduceOp.MAX)
             e2e = {"value": n_test / (float(ms2.item()) * 1e-3), "unit": "points/s",
                    "h2d_bytes_per_step": n_test * cfg["d"] * 8, "d2h_bytes_per_step": 2 * n_test * p * 8 + 8 * world}
+    dump = None
+    if keep is not None:
+        dump = host_outputs({"predict.mean": torch.cat(keep["mean"]), "predict.variance": torch.cat(keep["variance"])})
+        if world > 1:                                # the shards are contiguous and in rank order
+            shards = [None] * world
+            dist.all_gather_object(shards, dump)
+            dump = {k: torch.cat([s[k] for s in shards]) for k in dump}
     if rank == 0:
         peaks, peak_src = measured_peaks()
         main = products_per_fp64_product(eng)[0]
@@ -897,6 +982,8 @@ def run_predict_workload(args, cfg, world, rank, dev):
                                         % (i8_sus, i8_peak, main) if main else "live DMMA microbenchmark",
                          "fp64_dmma_peak": peak},
         }
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(line), flush=True)
 
 

@@ -6,6 +6,10 @@ import sys
 import types
 from pathlib import Path
 
+import numpy as np
+import pytest
+import torch
+
 import bench
 
 ROOT = Path(__file__).resolve().parents[1]
@@ -86,3 +90,44 @@ def test_reference_arm_prints_one_contract_line():
     assert line["impl"] == "reference" and line["cpu_baseline"]["kind"] == "port"
     assert "fitted_exponent" in line["cpu_baseline"] and line["cpu_baseline"]["samples_n_seconds"]
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0
+
+
+def test_steps_must_be_positive_and_set_the_count(monkeypatch, capsys):
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "5", "--warmup", "0"])
+    assert bench.parse().steps == 5
+    monkeypatch.setattr(sys, "argv", ["bench.py"])
+    assert bench.parse().steps is None                                    # the workload's own count
+    for bad in ("0", "-2"):
+        monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", bad])
+        with pytest.raises(SystemExit):
+            bench.parse()
+    assert "must be at least 1" in capsys.readouterr().err
+
+
+def test_dump_sample_is_fixed_sorted_and_fits_the_budget():
+    assert bench.sample_rows(1000, 80, 80 * 1000) is None                 # everything fits: no sampling
+    rows = bench.sample_rows(1000, 80, 8000)
+    assert rows.numel() == 100 and torch.equal(rows, bench.sample_rows(1000, 80, 8000))
+    assert torch.equal(rows, rows.unique()) and 0 <= rows.min() and rows.max() < 1000
+    assert bench.sample_rows(1000, 80, -5).numel() == 0
+
+
+def test_dump_writes_float_arrays_and_refuses_more_than_the_cap(tmp_path, monkeypatch):
+    arrays = bench.host_outputs({"loss": torch.tensor(1.5, dtype=torch.float64),
+                                 "param.a": torch.arange(6, dtype=torch.float32).reshape(2, 3),
+                                 "grad.b": torch.arange(4, dtype=torch.int64)})
+    bench.write_outputs(str(tmp_path / "out"), arrays)
+    loss, a, b = (np.load(tmp_path / "out" / f"{k}.npy") for k in ("loss", "param.a", "grad.b"))
+    assert loss.dtype == np.float64 and loss == 1.5
+    assert a.dtype == np.float32 and a.shape == (2, 3) and a[1, 2] == 5
+    assert b.dtype == np.float64 and b.tolist() == [0, 1, 2, 3]
+    monkeypatch.setattr(bench, "DUMP_BYTES", 16)
+    with pytest.raises(ValueError, match="cap"):
+        bench.write_outputs(str(tmp_path / "big"), arrays)
+    assert not (tmp_path / "big").exists()
+
+
+def test_reference_arm_refuses_to_dump_outputs(monkeypatch, tmp_path):
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--impl", "reference", "--dump-outputs", str(tmp_path)])
+    with pytest.raises(SystemExit, match="--impl ours"):
+        bench.main()
