@@ -219,6 +219,29 @@ int plmc_mix_tasks(const double* lat_mean, const double* lat_var, long long ldm,
                    const double* var_add, double* mean, double* var, long long mt, int p, int q, int accumulate,
                    void* stream);
 
+/* ---- joint predictive covariance and posterior draws (the full MultitaskMultivariateNormal of the eval branch,
+ * projected_lmc.py:1149-1155: covariance sum_l C_l (x) h_l h_l^T + eps I, + I (x) F F^T after full_likelihood).
+ * Latent posterior covariance C_l = K**_l - V_l^T V_l:  K**_l from plmc_gram on the scaled test points (diag_add 0),
+ * then  lower(C[l]) = alpha A[l]^T A[l] + beta C[l]  with A[l] = V_l [k, ldA] row-major (k rows, n columns),
+ * C [batch, n, ldc]; n % 128 == 0, k % 128 == 0.  One product per call, routed like the products of the factorisation
+ * (plmc_gemm_cfg: residue planes, digit planes or FP64 DMMA), the operand converted once (SYRK).                   */
+int plmc_syrk_batched(const double* A, long long lda, long long strideA, double* C, long long ldc, long long strideC,
+                      long long n, long long k, double alpha, double beta, int batch, const plmc_gemm_cfg* cfg,
+                      void* stream);
+/* T[(i,t),(j,s)] = sum_l C[l,i,j] H[l,t] H[l,s] + [i == j] S[t,s]   (point-major, task-minor; N = ns p)
+ * from the entries i >= j of C [q, >= ns, ldc] only; H [q, p] row-major; S [p, p] symmetric (T is then exactly
+ * symmetric).  tiled 0: T dense [N, ldt], ldt >= N;  tiled 1: the lower 128-tiles of a [npad(N), ldt] matrix with
+ * identity padding (the operand of plmc_potrf_batched, batch 1).  Writes 8 N^2 (about 4 npad(N)^2) bytes.           */
+int plmc_task_covariance(const double* C, long long ldc, long long stride, const double* H, const double* S,
+                         double* T, long long ldt, long long ns, int p, int q, int tiled, void* stream);
+/* out[s, j, t] = mean[j, t] + sum_l G[l, j, s] H[l, t] + sum_u E[s, j, u] R[t, u]
+ * mean [ns, p]; G [q, >= ns, ldg] latent draws (e.g. chol(C_l) eps_l from plmc_trmm_batched op 2, ldg >= S);
+ * H [q, p]; E [S, ns, p] standard normals; R [p, p] a root of the task-level noise (R R^T = S above);
+ * out [S, ns, p].  Each sample is written once.                                                                   */
+int plmc_mix_samples(const double* mean, const double* G, long long ldg, long long strideg, const double* H,
+                     const double* E, const double* R, double* out, long long ns, long long S, int p, int q,
+                     void* stream);
+
 /* ---- generic FP64 tensor-core GEMM (exposed for tests and roofline runs)
  * layout bit0: B(k,n) n-contiguous, bit1: A(m,k) m-contiguous (see gemm_dmma.cuh) */
 int plmc_gemm(int layout, const double* A, long long lda, long long sA, const double* B, long long ldb, long long sB,

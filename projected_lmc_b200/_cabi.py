@@ -67,6 +67,9 @@ _SIGNATURES = {
     "plmc_latent_mean": [P, LL, LL, P, LL, P, LL, LL, LL, I, P],
     "plmc_latent_var": [P, LL, LL, P, P, LL, LL, LL, I, P],
     "plmc_mix_tasks": [P, P, LL, P, P, P, P, LL, I, I, I, P],
+    "plmc_syrk_batched": [P, LL, LL, P, LL, LL, LL, LL, D, D, I, CFG, P],
+    "plmc_task_covariance": [P, LL, LL, P, P, P, LL, LL, I, I, I, P],
+    "plmc_mix_samples": [P, P, LL, LL, P, P, P, P, LL, LL, I, I, P],
     "plmc_gemm": [I, P, LL, LL, P, LL, LL, P, LL, LL, I, I, I, D, D, I, I, I, I, P],
     "plmc_ozaki_ws_bytes": [I, I, I, I, I],
     "plmc_rns_bits": [I, I],

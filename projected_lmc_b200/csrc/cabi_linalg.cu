@@ -191,6 +191,17 @@ int plmc_lauum_batched(double* L, long long ld, long long stride, long long npad
     return cx.status;
 }
 
+int plmc_syrk_batched(const double* A, long long lda, long long strideA, double* C, long long ldc, long long strideC,
+                      long long n, long long k, double alpha, double beta, int batch, const plmc_gemm_cfg* cfg,
+                      void* stream) {
+    if (!A || k <= 0 || (k % 128) || k > 2147483647LL || lda < n || (lda & 1) || bad_mat(C, ldc, n, batch))
+        return PLMC_ERR_BADARG;
+    LaCtx cx;
+    if (!make_ctx(cx, (cudaStream_t)stream, batch, cfg)) return PLMC_ERR_BADARG;
+    syrk_lower(cx, BMat{const_cast<double*>(A), lda, strideA}, (int)n, (int)k, BMat{C, ldc, strideC}, alpha, beta);
+    return cx.status;
+}
+
 int plmc_potri_batched(double* L, long long ld, long long stride, long long npad, int batch, double* dinv,
                        const plmc_gemm_cfg* cfg, void* stream) {
     if (bad_mat(L, ld, npad, batch) || !dinv) return PLMC_ERR_BADARG;

@@ -509,4 +509,10 @@ void lauum_lower(LaCtx& cx, BMat L, int n, DinvBuf D, long long blk0, bool fill_
     lauum_rec(cx, L, n, D, blk0);
 }
 
+// lower(C) := alpha A^T A + beta C  (A k x n): one routed product, the operand is converted once (same_operand)
+void syrk_lower(LaCtx& cx, BMat A, int n, int k, BMat C, double alpha, double beta) {
+    if (cx.status || n <= 0 || k <= 0) return;
+    gemm(cx, false, false, A, A, C, n, n, k, alpha, beta, /*lower=*/1);
+}
+
 }  // namespace plmc

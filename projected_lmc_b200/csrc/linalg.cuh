@@ -121,5 +121,7 @@ void trmm_lln_lower(LaCtx& cx, BMat X, int n, DinvBuf D, BMat B, int m, double a
 void trmm_lower(LaCtx& cx, int op, BMat X, int n, DinvBuf D, BMat B, int m, double alpha);
 // B := T^T * B  (T lower n x n, B n x m)
 void trmm_llt(LaCtx& cx, BMat T, int n, DinvBuf D, long long blk0, BMat B, int m);
+// lower(C) := alpha * A^T A + beta * C  (A k x n, C n x n), routed like every product of the recursions
+void syrk_lower(LaCtx& cx, BMat A, int n, int k, BMat C, double alpha, double beta);
 
 }  // namespace plmc

@@ -6,8 +6,10 @@
 // and the task mixing  mean[j,t] = sum_l m_l[j] H[l,t],
 //                      var [j,t] = sum_l v_l[j] H[l,t]^2 + eps (+ diag Sigma).
 // The reference materialises the full [q, n*, n*] posterior covariance and a
-// dense Kronecker sum (:1149-1153); only its diagonal is ever consumed
-// (.variance), so only the diagonal is computed here.
+// dense Kronecker sum (:1149-1153); .mean / .variance need only its diagonal,
+// which is what is computed here, eagerly and tiled over the test points.  The
+// joint quantities (covariance_matrix, rsample, log_prob) are computed on demand
+// from the latent blocks C_l = K**_l - V_l^T V_l by csrc/joint.cu.
 //
 // Kx / V are [q, npad, ldx] (train row, test column); the O(n^2 n*) part is the
 // TRSM (plmc_trsm_batched op 2) between the two reductions below.

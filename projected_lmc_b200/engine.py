@@ -290,33 +290,45 @@ class LatentEngine:
         if not bool(bad.any()):
             self.last_jitter = None
             return False
-        jitter = torch.zeros(q, dtype=torch.float64, device=noise.device)
+
+        def refactor(l, jitter):
+            sl = slice(l, l + 1)
+            da = (noise[sl] + jitter[sl]).contiguous()
+            self.generation += 1
+            self._gram_all(comps, scaled, da, K[sl], n, sl)
+            ops.potrf(K[sl], dinv[sl], info[sl], self.cfg_main)
+
+        # a failed member left garbage in its K; the others may have been overwritten by work queued after
+        # the factorisation (the inverse runs in place), so every member is rebuilt, jitter only where needed
+        self.last_jitter = self._jitter_retry(bad, info[:q], refactor, max_tries, rebuild_all_first=True)
+        return True
+
+    @staticmethod
+    def _jitter_retry(bad, info, refactor, max_tries, rebuild_all_first):
+        """psd_safe_cholesky's schedule after a failed batched factorisation (bad = host copy of info): jitter
+        cholesky_jitter * 10^i on the members that still fail, a RuntimeWarning per retry, NotPSDError at the end.
+        refactor(l, jitter) rebuilds member l with jitter[l] added to its diagonal and factorises it into info[l].
+        Returns the jitter per member."""
+        q = bad.shape[0]
+        jitter = torch.zeros(q, dtype=torch.float64, device=info.device)
         base = settings.cholesky_jitter.value()
         prev_bad = bad
         new = 0.0
-        # a failed member left garbage in its K; the others may have been overwritten by work queued after
-        # the factorisation (the inverse runs in place), so every member is rebuilt, jitter only where needed
-        first = True
+        first = rebuild_all_first
         for i in range(max_tries):
             new = base * (10**i)
             warnings.warn(f"A not p.d., added jitter of {new:.1e} to the diagonal", RuntimeWarning)
             members = range(q) if first else torch.nonzero(prev_bad).flatten().tolist()
             failing = set(torch.nonzero(prev_bad).flatten().tolist())
-            self.generation += 1
             for l in members:
                 if l in failing:
                     jitter[l] = new
-                sl = slice(l, l + 1)
-                da = (noise[sl] + jitter[sl]).contiguous()
-                self._gram_all(comps, scaled, da, K[sl], n, sl)
-                ops.potrf(K[sl], dinv[sl], info[sl], self.cfg_main)
+                refactor(l, jitter)
             first = False
-            now = info[:q].cpu()
             # members that were fine stay fine (same matrix); only previously failing ones can still fail
-            prev_bad = now
+            prev_bad = info.cpu()
             if not bool(prev_bad.any()):
-                self.last_jitter = jitter
-                return True
+                return jitter
         raise NotPSDError(f"Matrix not positive definite after repeatedly adding jitter up to {new:.1e}.")
 
     def _gram_potrf(self, ws, comps, scaled, noise, n, max_tries):
@@ -600,17 +612,123 @@ class LatentEngine:
             if Kx is None or Kx.shape[2] != mt:
                 Kx = None
                 Kx = torch.empty((q, np_, mt), dtype=torch.float64, device=dev)
-            xs = Xs[s0:s0 + cnt]
-            for g, ((kid, dims, ell, os_), (Z, zn, _, xm)) in enumerate(zip(st["comps"], st["scaled"])):
-                xg = xs if len(dims) == xs.shape[1] and tuple(dims) == tuple(range(xs.shape[1])) else \
-                    xs.index_select(1, torch.as_tensor(list(dims), device=dev))
-                Zt, znt = ops.scale_inputs(xg.contiguous(), xm, ell, mt)
-                ops.cross_gram(Z, zn, Zt, znt, kid, os_, Kx, n, mt, accumulate=(g > 0))
-            lat_mean[:, s0:s0 + cnt] = ops.latent_mean(Kx, st["alpha"], n, mt)[:, :cnt]
+            lat_mean[:, s0:s0 + cnt] = self._cross_mean_v(st, Xs[s0:s0 + cnt], Kx, mt, inverted, need_var)[:, :cnt]
             if need_var:
-                if inverted:
-                    ops.trmm(2, st["L"], st["dinv"], Kx, 1.0, self.cfg_main)
-                else:
-                    ops.trsm(2, st["L"], st["dinv"], Kx, 1.0, self.cfg_main)
                 lat_var[:, s0:s0 + cnt] = ops.latent_var(Kx, st["prior_var"], mt)[:, :cnt]
         return lat_mean, lat_var
+
+    @staticmethod
+    def _component_inputs(xs, dims):
+        if len(dims) == xs.shape[1] and tuple(dims) == tuple(range(xs.shape[1])):
+            return xs
+        return xs.index_select(1, torch.as_tensor(list(dims), device=xs.device)).contiguous()
+
+    def _cross_mean_v(self, st, xs, Kx, mt, inverted, need_v, zero_padding=False):
+        """Cross-Gram K* of the test points xs into Kx [q, npad, mt], the latent means K*^T alpha [q, mt] (returned)
+        and, if need_v, V = L^-1 K* in place (trmm by the explicit inverse once the state is inverted, else trsm).
+        zero_padding: the columns of the padding test points are zeroed before the solve, so that V^T V has
+        exact zeros outside the ns x ns block."""
+        n = st["n"]
+        for g, ((kid, dims, ell, os_), (Z, zn, _, xm)) in enumerate(zip(st["comps"], st["scaled"])):
+            Zt, znt = ops.scale_inputs(self._component_inputs(xs, dims), xm, ell, mt)
+            ops.cross_gram(Z, zn, Zt, znt, kid, os_, Kx, n, mt, accumulate=(g > 0))
+        lat_mean = ops.latent_mean(Kx, st["alpha"], n, mt)
+        if need_v:
+            if zero_padding:
+                Kx[:, :, xs.shape[0]:].zero_()
+            if inverted:
+                ops.trmm(2, st["L"], st["dinv"], Kx, 1.0, self.cfg_main)
+            else:
+                ops.trsm(2, st["L"], st["dinv"], Kx, 1.0, self.cfg_main)
+        return lat_mean
+
+    # -- joint posterior (full covariance, draws, joint log-density) -------------------------------------------
+    # The n* test points are one tile; every buffer below belongs to the joint computation (the factor in ws["K"],
+    # its dinv and the prediction state are only read).
+    def latent_covariance(self, st, Xs):
+        """Latent posterior means [q, n*] and covariances C = K** - V^T V as the lower 128-tiles of [q, m, m]
+        (m = npad(n*), identity padding)."""
+        q, n = st["q"], st["n"]
+        np_ = st["L"].shape[1]
+        ns = Xs.shape[0]
+        dev = Xs.device
+        if not self.state_is_current(st):
+            raise RuntimeError("stale prediction state: the engine workspace was rewritten after factorize()")
+        self._configure_fp64(dev, np_, q)
+        m = _npad(ns)
+        inverted = self._maybe_invert(st, ns)
+        V = torch.empty((q, np_, m), dtype=torch.float64, device=dev)
+        lat_mean = self._cross_mean_v(st, Xs, V, m, inverted, True, zero_padding=True)[:, :ns].contiguous()
+        C = torch.empty((q, m, m), dtype=torch.float64, device=dev)
+        zero = torch.zeros(q, dtype=torch.float64, device=dev)
+        for g, ((kid, dims, ell, os_), (_, _, _, xm)) in enumerate(zip(st["comps"], st["scaled"])):
+            Zs, zns = ops.scale_inputs(self._component_inputs(Xs, dims), xm, ell, m)
+            ops.gram(Zs, zns, kid, os_, zero, C, ns, accumulate=(g > 0))
+        ops.syrk(V, C, -1.0, 1.0, self.cfg_main)
+        return lat_mean, C
+
+    def factor_covariance(self, C, ns, max_tries=None):
+        """Lower Cholesky factors of the latent covariances C [q, m, m] (a new tensor; C is kept), with
+        psd_safe_cholesky's jitter schedule on the latents whose factorisation fails."""
+        if max_tries is None:
+            max_tries = settings.cholesky_max_tries.value()
+        q, m, _ = C.shape
+        Lc = C.clone()
+        dinv = ops.alloc_dinv(m, q, C.device)
+        info = torch.zeros(q, dtype=torch.int32, device=C.device)
+        ops.potrf(Lc, dinv, info, self.cfg_main)
+        bad = info.cpu()
+        if bool(bad.any()):
+            def refactor(l, jitter):
+                Lc[l].copy_(C[l])
+                Lc[l].diagonal()[:ns] += jitter[l]
+                ops.potrf(Lc[l:l + 1], dinv[l:l + 1], info[l:l + 1], self.cfg_main)
+
+            self._jitter_retry(bad, info, refactor, max_tries, rebuild_all_first=False)
+        return Lc, dinv
+
+    def latent_draws(self, Lc, dinv, normals):
+        """chol(C_l) eps_l for normals [q, n*, S]: [q, m, npad(S)] (rows >= n* and columns >= S are padding)."""
+        q, m, _ = Lc.shape
+        _, ns, S = normals.shape
+        G = torch.zeros((q, m, _npad(S)), dtype=torch.float64, device=Lc.device)
+        G[:, :ns, :S] = normals
+        ops.trmm(2, Lc, dinv, G, 1.0, self.cfg_main)
+        return G
+
+    def sample_latents(self, lat_mean, Lc, dinv, normals):
+        """Latent posterior draws mean_l + chol(C_l) eps_l: [q, n*, S] for given normals [q, n*, S]."""
+        ns, S = normals.shape[1], normals.shape[2]
+        return self.latent_draws(Lc, dinv, normals)[:, :ns, :S] + lat_mean[:, :, None]
+
+    def joint_log_prob(self, C, H, S, mean, values, max_tries=None):
+        """log N(values; mean, sum_l C_l (x) h_l h_l^T + I (x) S) for values [B, n*, p] (mean [n*, p]): [B]."""
+        if max_tries is None:
+            max_tries = settings.cholesky_max_tries.value()
+        B, ns, p = values.shape
+        N = ns * p
+        T = ops.task_covariance(C, H, S, ns, tiled=True)
+        T0 = T.clone()
+        Np = T.shape[1]
+        dinv = ops.alloc_dinv(Np, 1, T.device)
+        info = torch.zeros(1, dtype=torch.int32, device=T.device)
+        ops.potrf(T, dinv, info, self.cfg_main)
+        bad = info.cpu()
+        if bool(bad.any()):
+            def refactor(l, jitter):
+                T.copy_(T0)
+                T[0].diagonal()[:N] += jitter[0]
+                ops.potrf(T, dinv, info, self.cfg_main)
+
+            self._jitter_retry(bad, info, refactor, max_tries, rebuild_all_first=False)
+        del T0
+        resid = (values - mean).reshape(B, N)
+        if B == 1:
+            z, _, quad, logdet = ops.solve_logdet(T, dinv, resid.contiguous(), N)
+        else:
+            Z = torch.zeros((1, Np, _npad(B)), dtype=torch.float64, device=T.device)
+            Z[0, :N, :B] = resid.T
+            ops.trsm(2, T, dinv, Z, 1.0, self.cfg_main)
+            quad = Z[0, :N, :B].pow(2).sum(0)
+            logdet = 2.0 * T[0].diagonal()[:N].log().sum()
+        return -0.5 * (quad + logdet + N * math.log(2 * math.pi))

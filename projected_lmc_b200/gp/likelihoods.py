@@ -72,7 +72,7 @@ class MultitaskGaussianLikelihood(Likelihood):
         return Fm @ Fm.transpose(-1, -2)
 
     def forward(self, dist, *params, **kwargs):
-        return dist.add_task_noise(self.task_noise_covar.diagonal())
+        return dist.add_task_noise(self.task_noise_covar)
 
     def __call__(self, dist, *params, **kwargs):
         return self.forward(dist, *params, **kwargs)

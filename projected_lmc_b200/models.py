@@ -405,8 +405,12 @@ class ProjectedGPModel(ExactGPModel):
         if x.shape != tx.shape or not torch.equal(x, tx):
             raise RuntimeError("You must train on the training inputs!")
 
+    def _parameter_key(self):
+        """Changes whenever a parameter, train_y or the owned latent range changes."""
+        return tuple((id(p), p._version) for p in self.parameters()) + (self.train_y._version, self._latent_range)
+
     def _prediction_state(self):
-        key = tuple((id(p), p._version) for p in self.parameters()) + (self.train_y._version, self._latent_range)
+        key = self._parameter_key()
         # the factor lives in the engine's shared workspace: compute_loo / kernel_cond / a training-mode handle
         # rewrite it, so the cache is also checked against the engine's workspace generation
         stale = self._inducing() is None and not self._engine.state_is_current(self._pred_cache)
@@ -449,7 +453,7 @@ class ProjectedGPModel(ExactGPModel):
             st = self._prediction_state()
             xs = _as_f64(x if x.dim() > 1 else x.unsqueeze(-1)).contiguous()
             m, v = self._predict_latents(st, xs)
-        return LatentPosterior(m.to(x.dtype), v.to(x.dtype))
+        return LatentPosterior(m.to(x.dtype), v.to(x.dtype), _JointPosterior(self, xs, x.dtype))
 
     def kernel_cond(self):
         """Condition numbers of the noisy latent train covariances K_l + s_l I (dense SVD: small n)."""
@@ -481,6 +485,7 @@ class ProjectedGPModel(ExactGPModel):
         with torch.no_grad():
             st = self._prediction_state()
             xs = _as_f64(x if x.dim() > 1 else x.unsqueeze(-1)).contiguous()
+            joint = _JointPosterior(self, xs, x.dtype)
             # a non-finite test point gives NaN predictions for that point in the reference; the integer tensor
             # path of the solve would not propagate it, so such rows are computed at 0 and overwritten below
             bad_rows = ~torch.isfinite(xs).all(dim=1)
@@ -505,7 +510,9 @@ class ProjectedGPModel(ExactGPModel):
             if has_bad:
                 mean[bad_rows] = float("nan")
                 var[bad_rows] = float("nan")
-        return gp.distributions.MultitaskMultivariateNormal(mean.to(x.dtype), var.to(x.dtype))
+            joint.task_mean = mean
+            task_noise = float(self.eps) * torch.eye(self.n_tasks, dtype=torch.float64, device=xs.device)
+        return gp.distributions.MultitaskMultivariateNormal(mean.to(x.dtype), var.to(x.dtype), joint, task_noise)
 
 
 class _StoredLoss:
@@ -517,12 +524,127 @@ class _StoredLoss:
 
 
 class LatentPosterior:
-    def __init__(self, mean, variance):
+    def __init__(self, mean, variance, joint=None):
         self.mean, self.variance = mean, variance
+        self._joint = joint
+        self._covar = None
 
     @property
     def stddev(self):
         return self.variance.clamp_min(0).sqrt()
+
+    @property
+    def covariance_matrix(self):
+        """Latent posterior covariances [q, n*, n*] (the reference's batched latent MVN; computed on first access)."""
+        if self._covar is None:
+            self._covar = self._joint.latent_covariance()
+        return self._covar
+
+
+class _JointPosterior:
+    """The joint quantities of one eval-mode prediction, computed on demand: the latent posterior covariances
+    C_l = K**_l - V_l^T V_l, the task-level covariance, posterior draws and the joint log-density.  It keeps its own
+    copy of the test inputs and the parameter key of the prediction: a parameter or train_y changed since then is
+    an error, a rewritten engine workspace (compute_loo, a training step) only means the factor is recomputed."""
+
+    def __init__(self, model, xs, dtype):
+        self.model = model
+        self.xs = xs.clone()
+        self.bad_rows = ~torch.isfinite(self.xs).all(dim=1)
+        self.has_bad = bool(self.bad_rows.any())
+        if self.has_bad:        # computed at 0, reported as NaN (as the marginal variances)
+            self.xs[self.bad_rows] = 0.0
+        self.dtype = dtype
+        self.key = model._parameter_key()
+        self.task_mean = None    # [n*, p] float64, set by the task-level prediction
+        self._lat = None
+        self._factor = None
+
+    def _latent(self):
+        m = self.model
+        if m._inducing() is not None:
+            raise NotImplementedError("joint posterior quantities (covariance_matrix, rsample, log_prob) are not "
+                                      "implemented for the inducing-point (SGPR) model")
+        if m._latent_range != (0, m.n_latents) or m._dist_group is not None:
+            raise NotImplementedError("joint posterior quantities (covariance_matrix, rsample, log_prob) are not "
+                                      "implemented for latent-sharded models (distributed.shard_latents)")
+        if m._parameter_key() != self.key:
+            raise RuntimeError("the model's parameters or train_y changed after this prediction was made; "
+                               "call the model again for the joint posterior")
+        if self._lat is None:
+            with torch.no_grad():
+                self._lat = m._engine.latent_covariance(m._prediction_state(), self.xs)
+        return self._lat
+
+    def _no_nan_inputs(self):
+        if self.has_bad:
+            from .engine import NanError
+            raise NanError("cholesky: the posterior covariance contains NaN (non-finite test inputs)")
+
+    def _mixing(self):
+        return _as_f64(self.model.lmc_coefficients()).detach().contiguous()
+
+    def latent_covariance(self):
+        _, C = self._latent()
+        ns = self.xs.shape[0]
+        Cn = C[:, :ns, :ns]
+        out = torch.tril(Cn) + torch.tril(Cn, -1).transpose(1, 2)
+        if self.has_bad:
+            out[:, self.bad_rows, :] = float("nan")
+            out[:, :, self.bad_rows] = float("nan")
+        return out.to(self.dtype)
+
+    def task_covariance(self, task_noise):
+        _, C = self._latent()
+        ns, p = self.xs.shape[0], self.model.n_tasks
+        with torch.no_grad():
+            S = (0.5 * (task_noise + task_noise.T)).contiguous()     # exactly symmetric, so is the result
+            T = ops.task_covariance(C, self._mixing(), S, ns)
+            if self.has_bad:
+                T4 = T.view(ns, p, ns, p)
+                T4[self.bad_rows] = float("nan")
+                T4[:, :, self.bad_rows] = float("nan")
+        return T.to(self.dtype)
+
+    def rsample(self, sample_shape, task_noise):
+        self._no_nan_inputs()
+        lat_mean, C = self._latent()
+        ns, p, q = self.xs.shape[0], self.model.n_tasks, C.shape[0]
+        eng = self.model._engine
+        with torch.no_grad():
+            if self._factor is None:
+                self._factor = eng.factor_covariance(C, ns)
+            S = int(torch.Size(sample_shape).numel())
+            dev = C.device
+            eps = torch.randn((q, ns, S), dtype=torch.float64, device=dev)
+            E = torch.randn((S, ns, p), dtype=torch.float64, device=dev)
+            R = torch.linalg.cholesky(0.5 * (task_noise + task_noise.T)).contiguous()
+            G = eng.latent_draws(*self._factor, eps)
+            out = ops.mix_samples(self.task_mean, G, self._mixing(), E, R, ns, S)
+        return out.reshape(*sample_shape, ns, p).to(self.dtype)
+
+    def sample_latents(self, normals):
+        """Latent draws mean_l + chol(C_l) normals_l for given normals [q, n*, S] (deterministic)."""
+        self._no_nan_inputs()
+        lat_mean, C = self._latent()
+        eng = self.model._engine
+        with torch.no_grad():
+            if self._factor is None:
+                self._factor = eng.factor_covariance(C, self.xs.shape[0])
+            return eng.sample_latents(lat_mean, *self._factor, _as_f64(normals).contiguous())
+
+    def log_prob(self, value, task_noise):
+        self._no_nan_inputs()
+        _, C = self._latent()
+        ns, p = self.xs.shape[0], self.model.n_tasks
+        if value.shape[-2:] != (ns, p):
+            raise ValueError(f"log_prob expects values of shape [..., {ns}, {p}], got {tuple(value.shape)}")
+        batch = value.shape[:-2]
+        with torch.no_grad():
+            vals = _as_f64(value).reshape(-1, ns, p)
+            S = (0.5 * (task_noise + task_noise.T)).contiguous()
+            lp = self.model._engine.joint_log_prob(C, self._mixing(), S, self.task_mean, vals)
+        return lp.reshape(batch).to(value.dtype)
 
 
 def ops_components(spec, tensors):

@@ -286,6 +286,36 @@ def mix_tasks(lat_mean, lat_var, H, var_add, mean, var, mt, accumulate=False):
 
 
 @_on_device
+def syrk(A, C, alpha=1.0, beta=0.0, cfg=None):
+    """lower(C[b]) = alpha A[b]^T A[b] + beta C[b] for A [batch, k, >=n], C [batch, n, ld] (n, k multiples of 128)."""
+    b, n, _ = C.shape
+    check(lib().plmc_syrk_batched(ptr(A), A.stride(1), A.stride(0), ptr(C), C.stride(1), C.stride(0), n, A.shape[1],
+                                  float(alpha), float(beta), b, _cfgp(cfg), stream()), "syrk")
+
+
+@_on_device
+def task_covariance(C, H, S, ns, tiled=False):
+    """Task-level covariance from the lower tiles of C [q, m, m]: dense [ns p, ns p], or (tiled) the lower 128-tiles of
+    a [1, npad(ns p), npad(ns p)] matrix with identity padding."""
+    q, p = H.shape
+    N = ns * p
+    T = torch.empty((1, npad(N), npad(N)) if tiled else (N, N), dtype=torch.float64, device=C.device)
+    check(lib().plmc_task_covariance(ptr(C), C.stride(1), C.stride(0), ptr(H), ptr(S), ptr(T), T.stride(-2), ns, p, q,
+                                     int(tiled), stream()), "task_covariance")
+    return T
+
+
+@_on_device
+def mix_samples(mean, G, H, E, R, ns, S):
+    """out [S, ns, p] = mean + (latent draws G [q, >=ns, >=S] mixed by H) + E R^T."""
+    q, p = H.shape
+    out = torch.empty((S, ns, p), dtype=torch.float64, device=G.device)
+    check(lib().plmc_mix_samples(ptr(mean), ptr(G), G.stride(1), G.stride(0), ptr(H), ptr(E), ptr(R), ptr(out), ns, S,
+                                 p, q, stream()), "mix_samples")
+    return out
+
+
+@_on_device
 def peak_dmma(blocks, threads, iters, scratch):
     check(lib().plmc_peak_dmma(blocks, threads, iters, ptr(scratch), stream()), "peak_dmma")
     return blocks * (threads // 32) * iters * 16 * 512
