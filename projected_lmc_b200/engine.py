@@ -64,6 +64,7 @@ class LatentEngine:
         self._cfg = (None, None)
         self._cfg_key = None
         self._pinned = None
+        self._force_eager = False
         self._xsub = {}
         self._graphs = {}
         self.last_jitter = None
@@ -211,6 +212,10 @@ class LatentEngine:
             self._xsub = {}
         return self._xmean
 
+    def _forget_inputs(self):
+        """Drops what was derived from the contents of the inputs (column means, per-component input subsets)."""
+        self._xmean_key, self._xsub = None, {}
+
     def _sub_inputs(self, X, dims):
         """(X[:, dims] contiguous, its column means) for one component of an additive kernel (cached with X)."""
         full = self.xmean(X)
@@ -250,7 +255,9 @@ class LatentEngine:
     # cholesky_ex) and a finite-inputs flag are copied to pinned memory behind the factorisation and an event is
     # recorded.  The caller queues everything that follows (solves, inverse, sweep) and only then waits for that
     # event, so the GPU queue never drains; the jitter retry -- the rare path -- re-runs synchronously.
-    def _gram_potrf_launch(self, ws, comps, scaled, noise, n):
+    def _launch_factorisation(self, ws, comps, scaled, noise, n):
+        """Gram -> potrf of every latent in ws; info[:q] = first bad pivot, info[q] = non-finite-input flag.  Only
+        queues device work, so graph 1 of the graphed step captures this same call."""
         q = noise.shape[0]
         K, dinv, info = ws["K"], ws["dinv"], ws["info"]
         # psd_safe_cholesky refuses a matrix with NaN entries before it factors anything.  Every entry of K is a
@@ -266,23 +273,25 @@ class LatentEngine:
         self._mark("gram")
         ops.potrf(K, dinv, info[:q], self.cfg_main)
         info[q:] = (~finite).to(torch.int32)
-        if self.capture_mode:
-            return None
-        if self._pinned is None or self._pinned.numel() != q + 1:
-            self._pinned = torch.empty((q + 1,), dtype=torch.int32).pin_memory()
+
+    def _status_copy(self, info):
+        """Copies info into the engine's pinned buffer behind the queued work and records an event: (event, host
+        view), the view valid once the event has completed."""
+        if self._pinned is None or self._pinned.numel() != info.numel():
+            self._pinned = torch.empty((info.numel(),), dtype=torch.int32).pin_memory()
         self._pinned.copy_(info, non_blocking=True)
         ev = torch.cuda.Event()
         ev.record()
-        self._mark("potrf")
-        return ev
+        return ev, self._pinned
 
-    def _gram_potrf_resolve(self, ev, ws, comps, scaled, noise, n, max_tries):
-        """Wait for the factorisation's status; returns True if a jitter retry re-factorised K (everything
-        queued after the first attempt must then be redone)."""
+    def _resolve_factorisation(self, status, ws, comps, scaled, noise, n, max_tries):
+        """Wait for the factorisation's status (from _status_copy); returns True if a jitter retry re-factorised K
+        (everything queued after the first attempt must then be redone)."""
         q = noise.shape[0]
         K, dinv, info = ws["K"], ws["dinv"], ws["info"]
+        ev, host = status
         ev.synchronize()
-        host = self._pinned.clone()
+        host = host.clone()
         if int(host[q]) != 0:
             raise NanError("cholesky: the kernel matrix contains NaN (non-finite inputs, lengthscales, outputscale "
                            "or noise)")
@@ -331,10 +340,6 @@ class LatentEngine:
                 return jitter
         raise NotPSDError(f"Matrix not positive definite after repeatedly adding jitter up to {new:.1e}.")
 
-    def _gram_potrf(self, ws, comps, scaled, noise, n, max_tries):
-        ev = self._gram_potrf_launch(ws, comps, scaled, noise, n)
-        self._gram_potrf_resolve(ev, ws, comps, scaled, noise, n, max_tries)
-
     # -- training: log-probabilities and all partial gradients -------------------
     def log_prob_and_grads(self, X, TY, comps, noise, need_grad, max_tries=None):
         """lp [q] = log N(TY_l; 0, sum_g o_gl k_gl(X,X) + noise_l I) for comps = [(kernel id, dims, ell [q, d_g],
@@ -346,74 +351,79 @@ class LatentEngine:
         ws = self.workspace(X.device, q, n)
         np_ = ws["K"].shape[1]
         if need_grad and self.profile is None and 0 < np_ <= self.graph_max_order and X.is_cuda \
-                and not self.capture_mode:
-            return self._log_prob_and_grads_graphed(ws, X, TY, comps, noise, max_tries)
-        mark = self._mark
-        mark("start")
+                and not self.capture_mode and not self._force_eager:
+            key = (X.data_ptr(), X._version, tuple(X.shape), q, tuple((kid, tuple(dims), os_ is not None)
+                                                                      for kid, dims, ell, os_ in comps), self._cfg_key)
+            if key in self._graphs:
+                return self._log_prob_and_grads_graphed(ws, key, X, TY, comps, noise, max_tries)
+            # the first call with these inputs, kernel structure and arithmetic runs eagerly (lazy library
+            # initialisation must not happen under capture); the next one captures
+            self._graphs[key] = "warm"
+        self._mark("start")
         scaled = self._scaled(X, comps, np_)
-        ev = self._gram_potrf_launch(ws, comps, scaled, noise, n)
-        K, dinv = ws["K"], ws["dinv"]
-
-        def rest():
-            # z, alpha, the quadratic form and the log-determinant come from L itself (two HBM-bound block
-            # substitutions, csrc/trsv.cu) at full FP64-grade accuracy.  The explicit inverse K^-1 = L^-T L^-1
-            # (trtri + lauum, 2/3 of the flops of the iteration) then feeds ONLY the gradient sweep
-            # tr((alpha alpha^T - K^-1) dK), so both steps may run at the reduced cfg_kinv precision.
-            z, alpha, quad, logdet = ops.solve_logdet(K, dinv, TY, n, ws["rhs"])
-            lp = -0.5 * (quad + logdet + n * math.log(2 * math.pi))
-            mark("solve_logdet")
-            if not need_grad:
-                return lp, None
-            self.generation += 1
-            ops.trtri(K, dinv, self.cfg_kinv)
-            ops.lauum(K, dinv, self.cfg_kinv)
-            mark("potri")
-            g_noise, g_tensors = None, []
-            for (kid, dims, ell, os_), (Z, zn, _, _) in zip(comps, scaled):   # one sweep of K^-1 per additive component
-                g_ell, g_os, g_n = ops.grad_sweep(K, alpha, Z, zn, ell, kid, os_, n)
-                g_noise = g_n if g_noise is None else g_noise
-                g_tensors.append(g_ell)
-                if os_ is not None:
-                    g_tensors.append(g_os)
-            mark("grad_sweep")
-            return lp, (-alpha, g_noise, g_tensors)
-
-        out = rest()                      # queued behind the factorisation before its status is known
+        self._launch_factorisation(ws, comps, scaled, noise, n)
         if self.capture_mode:
             # the caller captures the whole training step into a CUDA graph (training.fit): no host wait in here;
             # it reads ws["info"] (first bad pivot per latent + the non-finite flag) after every replay and
             # repeats a failed iteration eagerly, where the jitter retry below applies
             self.capture_info = ws["info"]
-            return out
-        if self._gram_potrf_resolve(ev, ws, comps, scaled, noise, n, max_tries):
-            mark("retry")
-            out = rest()                  # a jitter retry re-factorised K: redo what depended on it
+            return self._solve_inverse_sweep(ws, comps, scaled, TY, n, need_grad)
+        status = self._status_copy(ws["info"])
+        self._mark("potrf")
+        # queued behind the factorisation before its status is known
+        out = self._solve_inverse_sweep(ws, comps, scaled, TY, n, need_grad)
+        if self._resolve_factorisation(status, ws, comps, scaled, noise, n, max_tries):
+            self._mark("retry")
+            # a jitter retry re-factorised K: redo what depended on it
+            out = self._solve_inverse_sweep(ws, comps, scaled, TY, n, need_grad)
         return out
 
+    def _solve_inverse_sweep(self, ws, comps, scaled, TY, n, need_grad):
+        """The step behind the factorisation in ws: (lp, None) or (lp, (dlp/dTY, dlp/dnoise, [dlp/dell_0, (dlp/dos_0),
+        ...])).  Only queues device work, so graph 2 of the graphed step captures this same call."""
+        # z, alpha, the quadratic form and the log-determinant come from L itself (two HBM-bound block
+        # substitutions, csrc/trsv.cu) at full FP64-grade accuracy.  The explicit inverse K^-1 = L^-T L^-1
+        # (trtri + lauum, 2/3 of the flops of the iteration) then feeds ONLY the gradient sweep
+        # tr((alpha alpha^T - K^-1) dK), so both steps may run at the reduced cfg_kinv precision.
+        K, dinv = ws["K"], ws["dinv"]
+        z, alpha, quad, logdet = ops.solve_logdet(K, dinv, TY, n, ws["rhs"])
+        lp = -0.5 * (quad + logdet + n * math.log(2 * math.pi))
+        self._mark("solve_logdet")
+        if not need_grad:
+            return lp, None
+        self.generation += 1
+        ops.trtri(K, dinv, self.cfg_kinv)
+        ops.lauum(K, dinv, self.cfg_kinv)
+        self._mark("potri")
+        g_noise, g_tensors = None, []
+        for (kid, dims, ell, os_), (Z, zn, _, _) in zip(comps, scaled):   # one sweep of K^-1 per additive component
+            g_ell, g_os, g_n = ops.grad_sweep(K, alpha, Z, zn, ell, kid, os_, n)
+            g_noise = g_n if g_noise is None else g_noise
+            g_tensors.append(g_ell)
+            if os_ is not None:
+                g_tensors.append(g_os)
+        self._mark("grad_sweep")
+        return lp, (-alpha, g_noise, g_tensors)
+
+    @contextlib.contextmanager
+    def _forced_eager(self):
+        """Steps inside the block run on the eager path, never through the engine-level CUDA graphs."""
+        was, self._force_eager = self._force_eager, True
+        try:
+            yield
+        finally:
+            self._force_eager = was
+
     # -- the same step as two replayed CUDA graphs (small problems) ---------------------------------------------
-    def _log_prob_and_grads_graphed(self, ws, X, TY, comps, noise, max_tries):
-        """Graph 1: scale -> Gram -> potrf -> status copy.  Graph 2: solves -> inverse -> sweep(s).  Inputs are copied
-        into static buffers, outputs cloned out of them; the status event sits between the two replays, so the
-        host waits for the factorisation only after the rest has been queued -- as in the eager path.  The first
-        call with a given (inputs, kernel structure, arithmetic) runs eagerly (lazy library initialisation must not
-        happen under capture), the second captures, later ones replay.  A failed factorisation falls back to the
-        eager retry loop."""
+    def _log_prob_and_grads_graphed(self, ws, key, X, TY, comps, noise, max_tries):
+        """Graph 1: scale -> Gram -> potrf.  Graph 2: solves -> inverse -> sweep(s).  Inputs are copied into static
+        buffers, outputs cloned out of them; the status copy sits between the two replays, so the host waits for
+        the factorisation only after the rest has been queued -- as in the eager path.  The call after the eager
+        warm-up of `key` captures, later ones replay.  A failed factorisation falls back to the eager retry loop."""
         n = X.shape[0]
-        q = noise.shape[0]
-        np_ = ws["K"].shape[1]
-        key = (X.data_ptr(), X._version, tuple(X.shape), q, tuple((kid, tuple(dims), os_ is not None)
-                                                                  for kid, dims, ell, os_ in comps), self._cfg_key)
-        st = self._graphs.get(key)
-        if st is None:                      # warm-up: eager, with graphs disabled for this one call
-            self._graphs[key] = "warm"
-            old = self.graph_max_order
-            self.graph_max_order = 0
-            try:
-                return self.log_prob_and_grads(X, TY, comps, noise, True, max_tries)
-            finally:
-                self.graph_max_order = old
+        st = self._graphs[key]
         if st == "warm":
-            st = self._capture(ws, X, TY, comps, noise, n, np_, q)
+            st = self._capture(ws, X, TY, comps, noise, n)
             self._graphs[key] = st
         # refresh the static inputs, replay
         st["TY"].copy_(TY)
@@ -424,70 +434,33 @@ class LatentEngine:
                 os_s.copy_(os_)
         self.generation += 1
         st["g1"].replay()
-        if self._pinned is None or self._pinned.numel() != q + 1:
-            self._pinned = torch.empty((q + 1,), dtype=torch.int32).pin_memory()
-        self._pinned.copy_(ws["info"], non_blocking=True)
-        ev = torch.cuda.Event()
-        ev.record()
+        status = self._status_copy(ws["info"])
         self.generation += 1
         st["g2"].replay()
         ops.stats_add(st["launches"])            # the library kernels inside the two graphs
-        lp, alpha, g_noise, g_tensors = st["out"]
-        out = (lp.clone(), (-alpha, g_noise.clone(), [g.clone() for g in g_tensors]))
-        scaled = st["scaled"]
-        if self._gram_potrf_resolve(ev, ws, st["comps"], scaled, st["noise"], n, max_tries):
+        lp, (neg_alpha, g_noise, g_tensors) = st["out"]
+        out = (lp.clone(), (neg_alpha.clone(), g_noise.clone(), [g.clone() for g in g_tensors]))
+        if self._resolve_factorisation(status, ws, st["comps"], st["scaled"], st["noise"], n, max_tries):
             # jitter retry re-factorised K eagerly: finish the step eagerly as well
-            K, dinv = ws["K"], ws["dinv"]
-            z, alpha, quad, logdet = ops.solve_logdet(K, dinv, TY, n, ws["rhs"])
-            lp = -0.5 * (quad + logdet + n * math.log(2 * math.pi))
-            self.generation += 1
-            ops.trtri(K, dinv, self.cfg_kinv)
-            ops.lauum(K, dinv, self.cfg_kinv)
-            g_noise, g_tensors = None, []
-            for (kid, dims, ell, os_), (Z, zn, _, _) in zip(st["comps"], scaled):
-                g_ell, g_os, g_n = ops.grad_sweep(K, alpha, Z, zn, ell, kid, os_, n)
-                g_noise = g_n if g_noise is None else g_noise
-                g_tensors.append(g_ell)
-                if os_ is not None:
-                    g_tensors.append(g_os)
-            out = (lp, (-alpha, g_noise, g_tensors))
+            out = self._solve_inverse_sweep(ws, st["comps"], st["scaled"], TY, n, True)
         return out
 
-    def _capture(self, ws, X, TY, comps, noise, n, np_, q):
-        dev = X.device
-        K, dinv, info = ws["K"], ws["dinv"], ws["info"]
+    def _capture(self, ws, X, TY, comps, noise, n):
         TY_s, noise_s = TY.clone(), noise.clone()
         params = [(ell.clone(), None if os_ is None else os_.clone()) for kid, dims, ell, os_ in comps]
         comps_s = [(kid, dims, e, o) for (kid, dims, _, _), (e, o) in zip(comps, params)]
         for kid, dims, _, _ in comps_s:
             self._sub_inputs(X, dims)            # column subsets / means are cached outside the graphs
-        torch.cuda.synchronize(dev)
+        torch.cuda.synchronize(X.device)
         g1, g2 = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
         launches0 = ops.stats_get()[0]
         with no_gc_during_capture(), torch.cuda.graph(g1):
-            scaled = self._scaled(X, comps_s, np_)
-            finite = torch.isfinite(noise_s).all()
-            for (kid, dims, ell, os_), (Z, zn, _, _) in zip(comps_s, scaled):
-                finite = finite & torch.isfinite(zn).all()
-                if os_ is not None:
-                    finite = finite & torch.isfinite(os_).all()
-            self._gram_all(comps_s, scaled, noise_s, K, n)
-            ops.potrf(K, dinv, info[:q], self.cfg_main)
-            info[q:] = (~finite).to(torch.int32)
+            scaled = self._scaled(X, comps_s, ws["K"].shape[1])
+            self._launch_factorisation(ws, comps_s, scaled, noise_s, n)
         with no_gc_during_capture(), torch.cuda.graph(g2, pool=g1.pool()):
-            z, alpha, quad, logdet = ops.solve_logdet(K, dinv, TY_s, n, ws["rhs"])
-            lp = -0.5 * (quad + logdet + n * math.log(2 * math.pi))
-            ops.trtri(K, dinv, self.cfg_kinv)
-            ops.lauum(K, dinv, self.cfg_kinv)
-            g_noise, g_tensors = None, []
-            for (kid, dims, ell, os_), (Z, zn, _, _) in zip(comps_s, scaled):
-                g_ell, g_os, g_n = ops.grad_sweep(K, alpha, Z, zn, ell, kid, os_, n)
-                g_noise = g_n if g_noise is None else g_noise
-                g_tensors.append(g_ell)
-                if os_ is not None:
-                    g_tensors.append(g_os)
-        return dict(g1=g1, g2=g2, TY=TY_s, noise=noise_s, params=params, comps=comps_s, scaled=scaled,
-                    out=(lp, alpha, g_noise, g_tensors), launches=ops.stats_get()[0] - launches0)
+            out = self._solve_inverse_sweep(ws, comps_s, scaled, TY_s, n, True)
+        return dict(g1=g1, g2=g2, TY=TY_s, noise=noise_s, params=params, comps=comps_s, scaled=scaled, out=out,
+                    launches=ops.stats_get()[0] - launches0)
 
     # -- optional phase timing (CUDA events on the launch stream; used by bench.py) --
     profile = None
@@ -522,33 +495,34 @@ class LatentEngine:
 
     # -- leave-one-out by-product (projected_lmc.py:1108-1119) ----------------------
     def loo(self, X, TY, comps, noise, max_tries=None):
-        if max_tries is None:
-            max_tries = settings.cholesky_max_tries.value()
-        n, d = X.shape
-        q = noise.shape[0]
-        ws = self.workspace(X.device, q, n)
-        np_ = ws["K"].shape[1]
-        scaled = self._scaled(X, comps, np_)
-        self._gram_potrf(ws, comps, scaled, noise, n, max_tries)
+        n = X.shape[0]
+        ws, _, alpha = self._factorise_and_solve(X, TY, comps, noise, max_tries)
         K, dinv = ws["K"], ws["dinv"]
-        _, alpha, _, _ = ops.solve_logdet(K, dinv, TY, n, ws["rhs"])
         self.generation += 1
         ops.potri(K, dinv, self.cfg_main)
         sigma2 = 1.0 / torch.diagonal(K, dim1=1, dim2=2)[:, :n]
         return sigma2, alpha * sigma2
 
+    def _factorise_and_solve(self, X, TY, comps, noise, max_tries):
+        """Gram -> potrf with the jitter retry -> alpha = K^-1 TY, synchronously: (ws, scaled inputs, alpha)."""
+        if max_tries is None:
+            max_tries = settings.cholesky_max_tries.value()
+        n = X.shape[0]
+        ws = self.workspace(X.device, noise.shape[0], n)
+        scaled = self._scaled(X, comps, ws["K"].shape[1])
+        self._launch_factorisation(ws, comps, scaled, noise, n)
+        status = self._status_copy(ws["info"])
+        self._mark("potrf")
+        self._resolve_factorisation(status, ws, comps, scaled, noise, n, max_tries)
+        _, alpha, _, _ = ops.solve_logdet(ws["K"], ws["dinv"], TY, n, ws["rhs"])
+        return ws, scaled, alpha
+
     # -- prediction -----------------------------------------------------------------
     def factorize(self, X, TY, comps, noise, max_tries=None):
         """Prediction cache: L (in ws['K']), dinv, alpha, scaled inputs of every kernel component."""
-        if max_tries is None:
-            max_tries = settings.cholesky_max_tries.value()
         n, d = X.shape
         q = noise.shape[0]
-        ws = self.workspace(X.device, q, n)
-        np_ = ws["K"].shape[1]
-        scaled = self._scaled(X, comps, np_)
-        self._gram_potrf(ws, comps, scaled, noise, n, max_tries)
-        _, alpha, _, _ = ops.solve_logdet(ws["K"], ws["dinv"], TY, n, ws["rhs"])
+        ws, scaled, alpha = self._factorise_and_solve(X, TY, comps, noise, max_tries)
         prior_var = None                      # k(x*, x*) = sum_g os_g k_g(0) = sum_g os_g (1 without a ScaleKernel)
         for kid, dims, ell, os_ in comps:
             v = torch.ones(q, dtype=torch.float64, device=X.device) if os_ is None else os_
@@ -561,6 +535,14 @@ class LatentEngine:
         shared workspace the prediction state points into."""
         return st is not None and st.get("generation") == self.generation and self._ws is not None and \
             st["L"].data_ptr() == self._ws["K"].data_ptr()
+
+    def _check_state(self, st, device):
+        """Refuses a stale prediction state and sets up the arithmetic for its order: (q, npad)."""
+        if not self.state_is_current(st):
+            raise RuntimeError("stale prediction state: the engine workspace was rewritten after factorize()")
+        q, np_ = st["q"], st["L"].shape[1]
+        self._configure_fp64(device, np_, q)
+        return q, np_
 
     @staticmethod
     def tile_points(q: int, np_: int, budget_bytes: int = None, device=None) -> int:
@@ -594,13 +576,9 @@ class LatentEngine:
 
     def predict_latents(self, st, Xs, need_var=True, tile=None):
         """Latent posterior means / variances at Xs: ([q, n*], [q, n*])."""
-        q, n = st["q"], st["n"]
-        np_ = st["L"].shape[1]
+        q, np_ = self._check_state(st, Xs.device)
         ns = Xs.shape[0]
         dev = Xs.device
-        if not self.state_is_current(st):
-            raise RuntimeError("stale prediction state: the engine workspace was rewritten after factorize()")
-        self._configure_fp64(dev, np_, q)
         mt_full = tile or self.tile_points(q, np_, device=dev)
         inverted = self._maybe_invert(st, ns) if need_var else False
         lat_mean = torch.empty((q, ns), dtype=torch.float64, device=dev)
@@ -648,13 +626,9 @@ class LatentEngine:
     def latent_covariance(self, st, Xs):
         """Latent posterior means [q, n*] and covariances C = K** - V^T V as the lower 128-tiles of [q, m, m]
         (m = npad(n*), identity padding)."""
-        q, n = st["q"], st["n"]
-        np_ = st["L"].shape[1]
+        q, np_ = self._check_state(st, Xs.device)
         ns = Xs.shape[0]
         dev = Xs.device
-        if not self.state_is_current(st):
-            raise RuntimeError("stale prediction state: the engine workspace was rewritten after factorize()")
-        self._configure_fp64(dev, np_, q)
         m = _npad(ns)
         inverted = self._maybe_invert(st, ns)
         V = torch.empty((q, np_, m), dtype=torch.float64, device=dev)
@@ -703,32 +677,18 @@ class LatentEngine:
 
     def joint_log_prob(self, C, H, S, mean, values, max_tries=None):
         """log N(values; mean, sum_l C_l (x) h_l h_l^T + I (x) S) for values [B, n*, p] (mean [n*, p]): [B]."""
-        if max_tries is None:
-            max_tries = settings.cholesky_max_tries.value()
         B, ns, p = values.shape
         N = ns * p
         T = ops.task_covariance(C, H, S, ns, tiled=True)
-        T0 = T.clone()
-        Np = T.shape[1]
-        dinv = ops.alloc_dinv(Np, 1, T.device)
-        info = torch.zeros(1, dtype=torch.int32, device=T.device)
-        ops.potrf(T, dinv, info, self.cfg_main)
-        bad = info.cpu()
-        if bool(bad.any()):
-            def refactor(l, jitter):
-                T.copy_(T0)
-                T[0].diagonal()[:N] += jitter[0]
-                ops.potrf(T, dinv, info, self.cfg_main)
-
-            self._jitter_retry(bad, info, refactor, max_tries, rebuild_all_first=False)
-        del T0
+        L, dinv = self.factor_covariance(T, N, max_tries)
+        del T                                 # only the factor is used from here on
         resid = (values - mean).reshape(B, N)
         if B == 1:
-            z, _, quad, logdet = ops.solve_logdet(T, dinv, resid.contiguous(), N)
+            z, _, quad, logdet = ops.solve_logdet(L, dinv, resid.contiguous(), N)
         else:
-            Z = torch.zeros((1, Np, _npad(B)), dtype=torch.float64, device=T.device)
+            Z = torch.zeros((1, L.shape[1], _npad(B)), dtype=torch.float64, device=L.device)
             Z[0, :N, :B] = resid.T
-            ops.trsm(2, T, dinv, Z, 1.0, self.cfg_main)
+            ops.trsm(2, L, dinv, Z, 1.0, self.cfg_main)
             quad = Z[0, :N, :B].pow(2).sum(0)
-            logdet = 2.0 * T[0].diagonal()[:N].log().sum()
+            logdet = 2.0 * L[0].diagonal()[:N].log().sum()
         return -0.5 * (quad + logdet + N * math.log(2 * math.pi))

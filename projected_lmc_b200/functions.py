@@ -6,6 +6,20 @@ import torch
 from . import ops
 
 
+def ops_components(spec, tensors):
+    """[(kernel id, dims, ell, os | None)] from the flat (spec, tensors) form used across the autograd boundary."""
+    out, i = [], 0
+    for kid, dims, has_os in spec:
+        ell = tensors[i]
+        i += 1
+        os_ = None
+        if has_os:
+            os_ = tensors[i]
+            i += 1
+        out.append((kid, dims, ell, os_))
+    return out
+
+
 class ProjectData(torch.autograd.Function):
     """TY = T^T Y^T  (kernel 1).  Gradient flows to T only (Y is data)."""
 
@@ -33,15 +47,7 @@ class LatentLogProb(torch.autograd.Function):
     @staticmethod
     def forward(ctx, engine, X, spec, TY, noise, *tensors):
         need = any(t is not None and t.requires_grad for t in (TY, noise, *tensors))
-        comps, i = [], 0
-        for kid, dims, has_os in spec:
-            ell = tensors[i].detach().contiguous()
-            i += 1
-            os_ = None
-            if has_os:
-                os_ = tensors[i].detach().contiguous()
-                i += 1
-            comps.append((kid, dims, ell, os_))
+        comps = ops_components(spec, [t.detach().contiguous() for t in tensors])
         lp, grads = engine.log_prob_and_grads(X, TY.detach().contiguous(), comps, noise.detach().contiguous(), need)
         ctx.grads = grads
         return lp

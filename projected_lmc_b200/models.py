@@ -20,7 +20,7 @@ from torch import Tensor
 
 from . import gp, ops
 from .engine import LatentEngine
-from .functions import LatentLogProb, ProjectData
+from .functions import LatentLogProb, ProjectData, ops_components
 from .mixing import (LMCMixingMatrix, LowerTriangularParam, PositiveDiagonalParam, ScalarParam,
                      UpperTriangularParam)
 
@@ -645,20 +645,6 @@ class _JointPosterior:
             S = (0.5 * (task_noise + task_noise.T)).contiguous()
             lp = self.model._engine.joint_log_prob(C, self._mixing(), S, self.task_mean, vals)
         return lp.reshape(batch).to(value.dtype)
-
-
-def ops_components(spec, tensors):
-    """[(kernel id, dims, ell, os | None)] from the flat (spec, tensors) form used across the autograd boundary."""
-    out, i = [], 0
-    for kid, dims, has_os in spec:
-        ell = tensors[i]
-        i += 1
-        os_ = None
-        if has_os:
-            os_ = tensors[i]
-            i += 1
-        out.append((kid, dims, ell, os_))
-    return out
 
 
 def _as_f64(t: Tensor) -> Tensor:

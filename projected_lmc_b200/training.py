@@ -31,7 +31,7 @@ from .engine import no_gc_during_capture
 
 def _invalidate_data_caches(eng, mll):
     """Forget everything derived from the contents of X and Y (column means, per-component input subsets, S = Y^T Y)."""
-    eng._xmean_key, eng._xsub = None, {}
+    eng._forget_inputs()
     if hasattr(mll, "_S_key"):
         mll._S_key = None
 
@@ -47,7 +47,6 @@ class _GraphedStep:
         self.params = [p for p in model.parameters() if p.requires_grad]
         dev = X.device
         self.it_t = torch.zeros(1, dtype=torch.long, device=dev)
-        self.pinned = None
         torch.cuda.synchronize(dev)
         self.g1, self.g2 = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
         optimizer.zero_grad(set_to_none=True)
@@ -90,13 +89,8 @@ class _GraphedStep:
             self.eng.capture_mode = False
         self.eng.generation += 2              # the replay rewrote the engine workspace (prediction caches)
         ops.stats_add(self.launches)
-        if self.pinned is None:
-            self.pinned = torch.empty((self.info.numel(),), dtype=torch.int32).pin_memory()
-        self.pinned.copy_(self.info, non_blocking=True)
-        ev = torch.cuda.Event()
-        ev.record()
+        ev, host = self.eng._status_copy(self.info)
         ev.synchronize()
-        host = self.pinned
         if int(host[-1]) != 0 or bool(host[:-1].any()):
             # failed factorisation (or non-finite inputs): repeat this iteration on the eager path, which applies
             # psd_safe_cholesky's jitter schedule (or raises NanError / NotPSDError); gradients go into the SAME
@@ -104,13 +98,9 @@ class _GraphedStep:
             for p in self.params:
                 if p.grad is not None:
                     p.grad.zero_()
-            old = self.eng.graph_max_order
-            self.eng.graph_max_order = 0
-            try:
+            with self.eng._forced_eager():
                 loss = -self.mll(self.model(self.X), self.Y)
                 loss.backward()
-            finally:
-                self.eng.graph_max_order = old
             self.hist[it] = loss.detach()
         self.g2.replay()
 
@@ -166,10 +156,8 @@ def fit(model, mll, X, Y, n_iter: int, lr: float = 1e-2, lr_min: Optional[float]
                 except Exception as ex:  # noqa: BLE001  (an op of this torch build that cannot be captured)
                     torch.cuda.synchronize(X.device)
                     can_graph, graph_note = False, repr(ex)[:200]
-                    if eng is not None:
-                        eng.capture_mode = False
-                        # what the aborted capture cached was recorded, never computed
-                        _invalidate_data_caches(eng, mll)
+                    # what the aborted capture cached was recorded, never computed
+                    _invalidate_data_caches(eng, mll)
                     warnings.warn("the training step could not be captured into a CUDA graph; continuing with eager "
                                   f"launches ({graph_note})", RuntimeWarning)
                     try:
