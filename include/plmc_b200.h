@@ -38,6 +38,12 @@ extern "C" {
 #define PLMC_KERNEL_MATERN52 1 /* (1+sqrt5 r+5/3 r^2) exp(-sqrt5 r)       */
 #define PLMC_KERNEL_MATERN32 2 /* (1+sqrt3 r) exp(-sqrt3 r)               */
 #define PLMC_KERNEL_MATERN12 3 /* exp(-r)                                 */
+#define PLMC_KERNEL_RQ 4       /* (1+s/(2 alpha))^-alpha, alpha per latent: gpytorch RQKernel */
+
+/* Kernels with a shape parameter (PLMC_KERNEL_RQ: alpha) are reached through the ...2 entry points, which take it
+ * as `shape` ([q], device, one value per latent) and return its gradient in `g_shape` ([q], may be NULL).  They
+ * return PLMC_ERR_BADARG for RQ with shape == NULL, for a non-NULL shape with kernels 0-3 and for g_shape without a
+ * shape.  The entry points without the 2 are these with shape = g_shape = NULL, result for result.              */
 
 /* ---- arithmetic of the large GEMMs of the factorisation layer (per call) ----------------------
  * FP64 matrix products with M, N and K all >= min_dim and M*N*K >= min_mnk can be computed on the tcgen05 INT8
@@ -122,6 +128,12 @@ int plmc_kernel_profile_host(int kernel_id, const double* s_host, long long n, d
 /* host-only helper: sqrt(s) and 1/sqrt(s) as the Cholesky leaf computes its pivots (one coupled Goldschmidt
  * iteration, csrc/kernel_math.cuh), for CPU-side accuracy tests; s <= 0 gives NaN for both. */
 int plmc_sqrt_reciprocal_host(const double* s_host, long long n, double* root_host, double* inv_host);
+/* host-only helper: k(s), dk/ds and dk/dshape (gpytorch RQKernel.forward and its autograd; 0 for kernels 0-3) with
+ * shape_host[i] the shape parameter of entry i (NULL for kernels 0-3). */
+int plmc_kernel_profile2_host(int kernel_id, const double* s_host, const double* shape_host, long long n,
+                              double* k_host, double* dk_host, double* dshape_host);
+/* host-only helper: log(1 + x), x >= 0, as the RQ kernel computes it on the device (torch.log1p in RQKernel) */
+int plmc_log1p_host(const double* x_host, long long n, double* out_host);
 /* xmean[k] = mean_i X[i,k] */
 int plmc_col_mean(const double* X, long long n, int d, double* xmean, void* stream);
 /* Z[l, i, k] = (X[i,k]-xmean[k]) / ell[l,k], zero padded to [q, rows_pad, dpad];
@@ -141,6 +153,15 @@ int plmc_cross_gram(const double* Ztrain, const double* zntrain, const double* Z
                     int kernel_id, const double* os, double* Kx, long long ldx, long long stride, long long n,
                     long long npad, long long mt_rows_pad, long long mt, int dpad, int q, int accumulate,
                     void* stream);
+/* plmc_gram / plmc_cross_gram with the kernel's shape parameter (RQKernel.forward under ScaleKernel, reached from
+ * projected_lmc.py:151-167 with kernel_type=RQKernel; the test-point block of exact_prediction likewise). */
+int plmc_gram2(const double* Z, const double* zn, int kernel_id, const double* os, const double* shape,
+               const double* diag_add, double* K, long long ld, long long stride, long long n, long long npad, int dpad,
+               int q, int accumulate, void* stream);
+int plmc_cross_gram2(const double* Ztrain, const double* zntrain, const double* Ztest, const double* zntest,
+                     int kernel_id, const double* os, const double* shape, double* Kx, long long ldx, long long stride,
+                     long long n, long long npad, long long mt_rows_pad, long long mt, int dpad, int q, int accumulate,
+                     void* stream);
 
 /* ---- adjoint of the cross-Gram block (inducing-point / SGPR variant: ExactGPModel(n_inducing_points=m),
  * projected_lmc.py:302-303 -> gpytorch InducingPointKernel).  Zr [q, rows_pad_r, dpad] / Zc [q, rows_pad_c, dpad]
@@ -153,6 +174,14 @@ int plmc_cross_gram_bwd(const double* Zr, long long rows_pad_r, const double* Zc
                         long long ldg, long long strideG, int kernel_id, const double* os, const double* ell,
                         double* g_ell, double* g_os, double* g_rows, double* partial, long long nr, long long nc, int d,
                         int dpad, int q, void* stream);
+/* with the kernel's shape parameter (autograd of RQKernel.forward inside InducingPointKernel): g_shape [q] = dL/dshape;
+ * partial: plmc_cross_gram_bwd_ws2(nr, nc, d, q, kernel_id) bytes */
+long long plmc_cross_gram_bwd_ws2(long long nr, long long nc, int d, int q, int kernel_id);
+int plmc_cross_gram_bwd2(const double* Zr, long long rows_pad_r, const double* Zc, long long rows_pad_c,
+                         const double* G, long long ldg, long long strideG, int kernel_id, const double* os,
+                         const double* shape, const double* ell, double* g_ell, double* g_os, double* g_shape,
+                         double* g_rows, double* partial, long long nr, long long nc, int d, int dpad, int q,
+                         void* stream);
 
 /* ---- (3) factorisation: MultivariateNormal.log_prob -> psd_safe_cholesky,
  * triangular solve, logdet (gpytorch; reached from projected_lmc.py:1201).     */
@@ -204,6 +233,14 @@ int plmc_grad_sweep(const double* Kinv, long long ld, long long stride, const do
                     const double* Z, const double* zn, const double* ell, int kernel_id, const double* os,
                     double* g_ell, double* g_os, double* g_noise, double* partial, long long n, long long npad, int d,
                     int dpad, int q, void* stream);
+/* with the kernel's shape parameter (loss.backward() through RQKernel.forward, experiments.py:270):
+ * g_shape[l] = sum W o dk/dshape, accumulated beside g_os in the same fixed order; partial: plmc_grad_ws2(npad, d, q,
+ * kernel_id) bytes */
+long long plmc_grad_ws2(long long npad, int d, int q, int kernel_id);
+int plmc_grad_sweep2(const double* Kinv, long long ld, long long stride, const double* alpha, long long lda_vec,
+                     const double* Z, const double* zn, const double* ell, int kernel_id, const double* os,
+                     const double* shape, double* g_ell, double* g_os, double* g_noise, double* g_shape,
+                     double* partial, long long n, long long npad, int d, int dpad, int q, void* stream);
 
 /* ---- prediction: eval ProjectedGPModel.__call__, projected_lmc.py:1121-1155 +
  * gpytorch exact_prediction.  Given V = L^-1 Kx (trsm op 2 applied to Kx):

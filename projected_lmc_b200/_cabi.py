@@ -47,6 +47,8 @@ _SIGNATURES = {
     "plmc_project_bwd_ws": [LL, I, I],
     "plmc_project_bwd": [P, P, LL, P, P, LL, I, I, P],
     "plmc_kernel_profile_host": [I, P, LL, P, P],
+    "plmc_kernel_profile2_host": [I, P, P, LL, P, P, P],
+    "plmc_log1p_host": [P, LL, P],
     "plmc_sqrt_reciprocal_host": [P, LL, P, P],
     "plmc_col_mean": [P, LL, I, P, P],
     "plmc_scale_inputs": [P, P, P, P, P, LL, I, I, LL, I, P],
@@ -54,6 +56,10 @@ _SIGNATURES = {
     "plmc_cross_gram": [P, P, P, P, I, P, P, LL, LL, LL, LL, LL, LL, I, I, I, P],
     "plmc_cross_gram_bwd_ws": [LL, LL, I, I],
     "plmc_cross_gram_bwd": [P, LL, P, LL, P, LL, LL, I, P, P, P, P, P, P, LL, LL, I, I, I, P],
+    "plmc_gram2": [P, P, I, P, P, P, P, LL, LL, LL, LL, I, I, I, P],
+    "plmc_cross_gram2": [P, P, P, P, I, P, P, P, LL, LL, LL, LL, LL, LL, I, I, I, P],
+    "plmc_cross_gram_bwd_ws2": [LL, LL, I, I, I],
+    "plmc_cross_gram_bwd2": [P, LL, P, LL, P, LL, LL, I, P, P, P, P, P, P, P, P, LL, LL, I, I, I, P],
     "plmc_potrf_batched": [P, LL, LL, LL, I, P, P, CFG, P],
     "plmc_trsm_batched": [I, P, LL, LL, LL, I, P, P, LL, LL, LL, D, CFG, P],
     "plmc_trmm_batched": [I, P, LL, LL, LL, I, P, P, LL, LL, LL, D, CFG, P],
@@ -64,6 +70,8 @@ _SIGNATURES = {
     "plmc_grad_ws": [LL, I, I],
     "plmc_sweep_debug": [I],
     "plmc_grad_sweep": [P, LL, LL, P, LL, P, P, P, I, P, P, P, P, P, LL, LL, I, I, I, P],
+    "plmc_grad_ws2": [LL, I, I, I],
+    "plmc_grad_sweep2": [P, LL, LL, P, LL, P, P, P, I, P, P, P, P, P, P, P, LL, LL, I, I, I, P],
     "plmc_latent_mean": [P, LL, LL, P, LL, P, LL, LL, LL, I, P],
     "plmc_latent_var": [P, LL, LL, P, P, LL, LL, LL, I, P],
     "plmc_mix_tasks": [P, P, LL, P, P, P, P, LL, I, I, I, P],
@@ -84,7 +92,7 @@ _SIGNATURES = {
     "plmc_peak_mixed": [I, I, LL, LL, P, P],
 }
 _RET_LL = {"plmc_npad", "plmc_dinv_bytes", "plmc_project_bwd_ws", "plmc_grad_ws", "plmc_ozaki_ws_bytes",
-           "plmc_rns_ws_bytes", "plmc_cross_gram_bwd_ws"}
+           "plmc_rns_ws_bytes", "plmc_cross_gram_bwd_ws", "plmc_grad_ws2", "plmc_cross_gram_bwd_ws2"}
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

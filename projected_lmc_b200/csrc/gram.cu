@@ -13,6 +13,7 @@
 //
 // Algorithmic bytes: 8*q*n(n+1)/2 written (Gram), the same read (sweep).
 #include "kernel_math.cuh"
+#include "plmc_b200.h"
 
 namespace plmc {
 
@@ -67,7 +68,8 @@ __global__ void __launch_bounds__(GR_THREADS, 2)
     gram_kernel(const double* __restrict__ Zr, const double* __restrict__ znr, long long rows_pad_r,
                 const double* __restrict__ Zc, const double* __restrict__ znc, long long rows_pad_c,
                 const double* __restrict__ os, const double* __restrict__ diag_add, double* __restrict__ Kout,
-                long long ld, long long stride, long long n, int dpad, int tiles_c, int accumulate) {
+                long long ld, long long stride, long long n, int dpad, int tiles_c, int accumulate,
+                const double* __restrict__ shape) {
     extern __shared__ __align__(16) double sm[];
     const int kcmax = gram_kc(dpad);
     const int lds = gram_lds(kcmax);
@@ -95,6 +97,7 @@ __global__ void __launch_bounds__(GR_THREADS, 2)
     const long long i0 = (long long)ti * 128, j0 = (long long)tj * 128;
     const double* zc = Zc + ((long long)l * rows_pad_c + j0) * dpad;
     const double osl = os ? os[l] : 1.0;
+    const KernelShape sh = (KID == 4) ? kernel_shape(shape[l]) : KernelShape{0.0, 0.0};
     const double dadd = (MODE == 0) ? diag_add[l] : 0.0;
     double* Kl = Kout + (long long)l * stride;
     const bool single = dpad <= kcmax;   // one chunk: the column side is staged once per tile
@@ -171,8 +174,8 @@ __global__ void __launch_bounds__(GR_THREADS, 2)
             for (int pr = 0; pr < 16; ++pr) {
                 const int i = pr >> 2, j = pr & 3;
                 double* dst = base + (long long)(i * 8) * ld + j * 8;
-                double v0 = osl * kernel_value<KID>(stage[(pr * 2 + 0) * GR_THREADS + tid]);
-                double v1 = osl * kernel_value<KID>(stage[(pr * 2 + 1) * GR_THREADS + tid]);
+                double v0 = osl * kernel_value<KID>(stage[(pr * 2 + 0) * GR_THREADS + tid], sh);
+                double v1 = osl * kernel_value<KID>(stage[(pr * 2 + 1) * GR_THREADS + tid], sh);
                 if (accumulate) {
                     const double2 old = *reinterpret_cast<const double2*>(dst);
                     v0 += old.x;
@@ -198,12 +201,12 @@ __global__ void __launch_bounds__(GR_THREADS, 2)
                 double s = stage[(pr * 2 + e) * GR_THREADS + tid];
                 if (MODE == 0) {
                     if (gi == gje) s = 0.0;
-                    double kv = osl * kernel_value<KID>(s);
+                    double kv = osl * kernel_value<KID>(s, sh);
                     if (gi == gje && !accumulate) kv += dadd;
                     if (gi >= n || gje >= n) kv = (gi == gje && !accumulate) ? 1.0 : 0.0;
                     v[e] = kv;
                 } else {
-                    v[e] = (gi < n) ? osl * kernel_value<KID>(s) : 0.0;
+                    v[e] = (gi < n) ? osl * kernel_value<KID>(s, sh) : 0.0;
                 }
             }
             *reinterpret_cast<double2*>(Kl + gi * ld + gj) = make_double2(v[0] + old.x, v[1] + old.y);
@@ -226,23 +229,24 @@ __global__ void __launch_bounds__(GR_THREADS, 1)
     grad_sweep_kernel(const double* __restrict__ Kinv, long long ld, long long stride,
                       const double* __restrict__ alpha, long long lda_vec, const double* __restrict__ Z,
                       const double* __restrict__ os, double* __restrict__ partial, long long n, long long npad,
-                      int dpad, long long ntiles) {
+                      int dpad, long long ntiles, const double* __restrict__ shape) {
     extern __shared__ __align__(16) double sm[];
     const int lds = dpad + 1;
     double* Zi = sm;                    // [128][lds]
     double* Zj = Zi + 128 * lds;        // [128][lds]
     double* ai = Zj + 128 * lds;        // [128]
     double* aj = ai + 128;              // [128]
-    double* wsum = aj + 128;            // [8][dpad+2]
-    double* cta_acc = wsum + 8 * (dpad + 2);  // [dpad+2]
-    double* stage = cta_acc + (dpad + 2);     // [64][256] private per-thread slots
+    double* wsum = aj + 128;            // [8][nacc]
+    double* cta_acc = wsum + 8 * (dpad + 2 + (KID == 4 ? 1 : 0));  // [nacc]
+    double* stage = cta_acc + (dpad + 2 + (KID == 4 ? 1 : 0));     // [64][256] private per-thread slots
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int g = lane >> 2, t = lane & 3;
     const int wm = warp >> 2, wn = warp & 3;
     const int l = blockIdx.z;
-    const int nacc = dpad + 2;
+    const int nacc = dpad + 2 + (KID == 4 ? 1 : 0);   // + sum w W dk/dalpha (RQ)
     const double osl = os ? os[l] : 1.0;
+    const KernelShape sh = (KID == 4) ? kernel_shape(shape[l]) : KernelShape{0.0, 0.0};
     const double* Kl = Kinv + (long long)l * stride;
     const double* al = alpha + (long long)l * lda_vec;
     const double* Zl = Z + (long long)l * npad * dpad;
@@ -300,7 +304,7 @@ __global__ void __launch_bounds__(GR_THREADS, 1)
         for (int i = 0; i < 8; ++i)
 #pragma unroll
             for (int c = 0; c < 8; ++c) stage[(i * 8 + c) * GR_THREADS + tid] = Wv[i][c];
-        double s_os = 0.0, s_tr = 0.0;
+        double s_os = 0.0, s_tr = 0.0, s_al = 0.0;
 #pragma unroll 4
         for (int pr = 0; pr < 32; ++pr) {
             const int i = pr >> 2, j = pr & 3;
@@ -315,9 +319,10 @@ __global__ void __launch_bounds__(GR_THREADS, 1)
                 double w = (gj < gi) ? 2.0 : (gj == gi ? 1.0 : 0.0);
                 if (gi >= n || gj >= n) w = 0.0;
                 const double Wij = (w != 0.0) ? 0.5 * (a_i * aj[cl] - (e ? kv.y : kv.x)) : 0.0;
-                double kk, dk;
-                kernel_value_grad<KID>(stage[(pr * 2 + e) * GR_THREADS + tid], kk, dk);
+                double kk, dk, dka;
+                kernel_value_grad<KID>(stage[(pr * 2 + e) * GR_THREADS + tid], kk, dk, dka, sh);
                 s_os = fma(w * Wij, kk, s_os);
+                if (KID == 4) s_al = fma(w * Wij, dka, s_al);
                 if (gj == gi && gi < n) s_tr += Wij;
                 stage[(pr * 2 + e) * GR_THREADS + tid] = w * Wij * osl * dk;
             }
@@ -349,9 +354,11 @@ __global__ void __launch_bounds__(GR_THREADS, 1)
         }
         s_os = warp_sum(s_os);
         s_tr = warp_sum(s_tr);
+        if (KID == 4) s_al = warp_sum(s_al);
         if (lane == 0) {
             wsum[warp * nacc + dpad] = s_os;
             wsum[warp * nacc + dpad + 1] = s_tr;
+            if (KID == 4) wsum[warp * nacc + dpad + 2] = s_al;
         }
         __syncthreads();
         if (tid < nacc) {
@@ -389,7 +396,8 @@ template <int KID, bool INTERIOR>
 __device__ __forceinline__ void sweep_transform(double* __restrict__ At, const double* __restrict__ aj,
                                                 const double* __restrict__ Kl, long long ld, long long ih0,
                                                 long long j0, long long n, int wm, int wn, int g, int t,
-                                                const double (&ai)[4], double osl, double& s_os, double& s_tr) {
+                                                const double (&ai)[4], double osl, double& s_os, double& s_tr,
+                                                KernelShape sh, double& s_al) {
 #pragma unroll 1
     for (int j = 0; j < 4; ++j) {
         const int cl = wn * 32 + j * 8 + 2 * t;
@@ -409,10 +417,11 @@ __device__ __forceinline__ void sweep_transform(double* __restrict__ At, const d
 #pragma unroll
             for (int e = 0; e < 2; ++e) {
                 const double raw = fma(ai[i], e ? ajv.y : ajv.x, -(e ? kv[i].y : kv[i].x));   // 2 W_ij
-                double kk, dk;
-                kernel_value_grad<KID>(e ? sv.y : sv.x, kk, dk);
+                double kk, dk, dka;
+                kernel_value_grad<KID>(e ? sv.y : sv.x, kk, dk, dka, sh);
                 if (INTERIOR) {                       // strictly below the diagonal, no padding: w/2 = 1
                     s_os = fma(raw, kk, s_os);
+                    if (KID == 4) s_al = fma(raw, dka, s_al);
                     out[e] = raw * (osl * dk);
                 } else {
                     const long long gje = gj + e;
@@ -420,6 +429,7 @@ __device__ __forceinline__ void sweep_transform(double* __restrict__ At, const d
                     if (gi >= n || gje >= n) w = 0.0;
                     const double c1 = (w != 0.0) ? w * raw : 0.0;   // entries above the diagonal are never used
                     s_os = fma(c1, kk, s_os);
+                    if (KID == 4) s_al = fma(c1, dka, s_al);
                     if (gje == gi) s_tr += c1;
                     out[e] = (gje == gi) ? 0.0 : c1 * (osl * dk);
                 }
@@ -434,7 +444,7 @@ __global__ void __launch_bounds__(GR_THREADS, 2)
     grad_sweep2_kernel(const double* __restrict__ Kinv, long long ld, long long stride,
                        const double* __restrict__ alpha, long long lda_vec, const double* __restrict__ Z,
                        const double* __restrict__ zn, const double* __restrict__ os, double* __restrict__ partial,
-                       long long n, long long npad, int dpad, long long ntiles) {
+                       long long n, long long npad, int dpad, long long ntiles, const double* __restrict__ shape) {
     extern __shared__ __align__(16) double sm[];
     const int lds = sweep_lds(dpad);
     double* Zj = sm;                     // [128][lds]
@@ -447,8 +457,9 @@ __global__ void __launch_bounds__(GR_THREADS, 2)
     const int g = lane >> 2, t = lane & 3;
     const int wm = warp >> 2, wn = warp & 3;
     const int l = blockIdx.z;
-    const int nacc = dpad + 2;
+    const int nacc = dpad + 2 + (KID == 4 ? 1 : 0);
     const double osl = os ? os[l] : 1.0;
+    const KernelShape sh = (KID == 4) ? kernel_shape(shape[l]) : KernelShape{0.0, 0.0};
     const double* Kl = Kinv + (long long)l * stride;
     const double* al = alpha + (long long)l * lda_vec;
     const double* Zl = Z + (long long)l * npad * dpad;
@@ -465,7 +476,7 @@ __global__ void __launch_bounds__(GR_THREADS, 2)
 #pragma unroll
     for (int nb = 0; nb < NB; ++nb) gacc[nb][0] = gacc[nb][1] = 0.0;
     double cacc = 0.0;                   // dim = lane, column-side term
-    double s_os = 0.0, s_tr = 0.0;
+    double s_os = 0.0, s_tr = 0.0, s_al = 0.0;   // s_al: sum w W dk/dalpha (RQ only)
 
     for (long long b = blockIdx.x; b < ntiles; b += gridDim.x) {
         int r = (int)((sqrt(8.0 * (double)b + 1.0) - 1.0) * 0.5);
@@ -540,9 +551,9 @@ __global__ void __launch_bounds__(GR_THREADS, 2)
             }
             // ---- 2. transform in place (a thread reads back only the slots it wrote: no barrier)
             if (interior)
-                sweep_transform<KID, true>(At, aj, Kl, ld, ih0, j0, n, wm, wn, g, t, ai, osl, s_os, s_tr);
+                sweep_transform<KID, true>(At, aj, Kl, ld, ih0, j0, n, wm, wn, g, t, ai, osl, s_os, s_tr, sh, s_al);
             else
-                sweep_transform<KID, false>(At, aj, Kl, ld, ih0, j0, n, wm, wn, g, t, ai, osl, s_os, s_tr);
+                sweep_transform<KID, false>(At, aj, Kl, ld, ih0, j0, n, wm, wn, g, t, ai, osl, s_os, s_tr, sh, s_al);
             __syncthreads();             // At = A complete
 
             // ---- 3. U = A Zj on DMMA (warp w: rows 8w..8w+7), row sums from the same fragments, column sums
@@ -608,9 +619,11 @@ __global__ void __launch_bounds__(GR_THREADS, 2)
     if (lane < NB * 8) red2[warp * (NB * 8) + lane] = cacc;
     s_os = warp_sum(s_os);
     s_tr = warp_sum(s_tr);
+    if (KID == 4) s_al = warp_sum(s_al);
     if (lane == 0) {
         red[warp * nacc + dpad] = s_os;
         red[warp * nacc + dpad + 1] = s_tr;
+        if (KID == 4) red[warp * nacc + dpad + 2] = s_al;
     }
     __syncthreads();
     if (tid < nacc) {
@@ -627,12 +640,13 @@ __global__ void __launch_bounds__(GR_THREADS, 2)
     }
 }
 
-// g_ell[l,k] = -(2/ell[l,k]) * sum_c partial[l,c,k] ; g_os, g_noise likewise
+// g_ell[l,k] = -(2/ell[l,k]) * sum_c partial[l,c,k] ; g_os, g_noise likewise; with a shape parameter (nacc =
+// dpad + 3) g_shape[l] = os[l] * sum_c partial[l,c,dpad+2]
 __global__ void grad_reduce_kernel(const double* __restrict__ partial, int chunks, int d, int dpad,
                                    const double* __restrict__ ell, double* __restrict__ g_ell,
-                                   double* __restrict__ g_os, double* __restrict__ g_noise) {
+                                   double* __restrict__ g_os, double* __restrict__ g_noise, int nacc,
+                                   const double* __restrict__ os, double* __restrict__ g_shape) {
     const int l = blockIdx.x;
-    const int nacc = dpad + 2;
     for (int a = threadIdx.x; a < nacc; a += blockDim.x) {
         double s = 0.0;
         for (int c = 0; c < chunks; ++c) s += partial[((long long)l * chunks + c) * nacc + a];
@@ -642,10 +656,17 @@ __global__ void grad_reduce_kernel(const double* __restrict__ partial, int chunk
             if (g_os) g_os[l] = s;
         } else if (a == dpad + 1)
             g_noise[l] = s;
+        else if (a == dpad + 2 && g_shape)
+            g_shape[l] = (os ? os[l] : 1.0) * s;
     }
 }
 
 static inline int sweep_ctas(long long ntiles) { return (int)(ntiles < 592 ? ntiles : 592); }
+
+// the shape argument of the ...2 entry points: required by RQ, refused by the kernels without a shape parameter
+static inline bool shape_arg_ok(int kernel_id, const double* shape) {
+    return (kernel_id == PLMC_KERNEL_RQ) == (shape != nullptr);
+}
 
 }  // namespace plmc
 
@@ -658,19 +679,20 @@ template <int MODE>
 static int launch_gram(int kernel_id, dim3 grid, size_t smem, cudaStream_t st, const double* Zr, const double* znr,
                        long long rpr, const double* Zc, const double* znc, long long rpc, const double* os,
                        const double* diag_add, double* K, long long ld, long long stride, long long n, int dpad,
-                       int tiles_c, int accumulate) {
+                       int tiles_c, int accumulate, const double* shape) {
 #define PLMC_GRAM_CASE(KID)                                                                                     \
     case KID:                                                                                                   \
         if (smem > 48 * 1024)                                                                                   \
             cudaFuncSetAttribute(gram_kernel<KID, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
         gram_kernel<KID, MODE><<<grid, GR_THREADS, smem, st>>>(Zr, znr, rpr, Zc, znc, rpc, os, diag_add, K, ld,  \
-                                                               stride, n, dpad, tiles_c, accumulate);           \
+                                                               stride, n, dpad, tiles_c, accumulate, shape);    \
         break;
     switch (kernel_id) {
         PLMC_GRAM_CASE(0)
         PLMC_GRAM_CASE(1)
         PLMC_GRAM_CASE(2)
         PLMC_GRAM_CASE(3)
+        PLMC_GRAM_CASE(4)
         default: return PLMC_ERR_BADARG;
     }
 #undef PLMC_GRAM_CASE
@@ -694,6 +716,33 @@ int plmc_kernel_profile_host(int kernel_id, const double* s_host, long long n, d
             default: return PLMC_ERR_BADARG;
         }
     }
+    return PLMC_OK;
+}
+
+/* host only: k(s), dk/ds and dk/dshape with the device source, shape[i] the kernel's shape parameter for s[i]
+ * (RQ: alpha; NULL for kernels 0-3, whose dk/dshape is 0) */
+int plmc_kernel_profile2_host(int kernel_id, const double* s_host, const double* shape_host, long long n,
+                              double* k_host, double* dk_host, double* dshape_host) {
+    if (!s_host || !k_host || !dk_host || !dshape_host || n < 0 || kernel_id < 0 || kernel_id > PLMC_KERNEL_RQ ||
+        !shape_arg_ok(kernel_id, shape_host))
+        return PLMC_ERR_BADARG;
+    for (long long i = 0; i < n; ++i) {
+        switch (kernel_id) {
+            case 0: kernel_value_grad<0>(s_host[i], k_host[i], dk_host[i], dshape_host[i], KernelShape{}); break;
+            case 1: kernel_value_grad<1>(s_host[i], k_host[i], dk_host[i], dshape_host[i], KernelShape{}); break;
+            case 2: kernel_value_grad<2>(s_host[i], k_host[i], dk_host[i], dshape_host[i], KernelShape{}); break;
+            case 3: kernel_value_grad<3>(s_host[i], k_host[i], dk_host[i], dshape_host[i], KernelShape{}); break;
+            default:
+                kernel_value_grad<4>(s_host[i], k_host[i], dk_host[i], dshape_host[i], kernel_shape(shape_host[i]));
+        }
+    }
+    return PLMC_OK;
+}
+
+/* host only: log1p(x), x >= 0, as the RQ kernel evaluates it on the device (csrc/kernel_math.cuh) */
+int plmc_log1p_host(const double* x_host, long long n, double* out_host) {
+    if (!x_host || !out_host || n < 0) return PLMC_ERR_BADARG;
+    for (long long i = 0; i < n; ++i) out_host[i] = log1p_nonneg(x_host[i]);
     return PLMC_OK;
 }
 
@@ -726,29 +775,45 @@ int plmc_scale_inputs(const double* X, const double* xmean, const double* ell, d
 int plmc_gram(const double* Z, const double* zn, int kernel_id, const double* os, const double* diag_add, double* K,
               long long ld, long long stride, long long n, long long npad, int dpad, int q, int accumulate,
               void* stream) {
+    return plmc_gram2(Z, zn, kernel_id, os, nullptr, diag_add, K, ld, stride, n, npad, dpad, q, accumulate, stream);
+}
+
+int plmc_gram2(const double* Z, const double* zn, int kernel_id, const double* os, const double* shape,
+               const double* diag_add, double* K, long long ld, long long stride, long long n, long long npad, int dpad,
+               int q, int accumulate, void* stream) {
     if (!Z || !zn || !diag_add || !K || n <= 0 || npad < n || (npad % 128) || ld < npad || (ld & 1) || dpad <= 0 ||
-        (dpad & 3) || q <= 0 || q > 65535)
+        (dpad & 3) || q <= 0 || q > 65535 || !shape_arg_ok(kernel_id, shape))
         return PLMC_ERR_BADARG;
     const long long tm = npad / 128;
     const long long tiles = tm * (tm + 1) / 2;
     if (tiles > 2147483647LL) return PLMC_ERR_BADARG;
     const size_t smem = gram_smem(dpad);
     return launch_gram<0>(kernel_id, dim3((unsigned)tiles, 1, q), smem, (cudaStream_t)stream, Z, zn, npad, Z, zn, npad,
-                          os, diag_add, K, ld, stride, n, dpad, (int)tm, accumulate);
+                          os, diag_add, K, ld, stride, n, dpad, (int)tm, accumulate, shape);
 }
 
 int plmc_cross_gram(const double* Ztrain, const double* zntrain, const double* Ztest, const double* zntest,
                     int kernel_id, const double* os, double* Kx, long long ldx, long long stride, long long n,
                     long long npad, long long mt_rows_pad, long long mt, int dpad, int q, int accumulate,
                     void* stream) {
+    return plmc_cross_gram2(Ztrain, zntrain, Ztest, zntest, kernel_id, os, nullptr, Kx, ldx, stride, n, npad,
+                            mt_rows_pad, mt, dpad, q, accumulate, stream);
+}
+
+int plmc_cross_gram2(const double* Ztrain, const double* zntrain, const double* Ztest, const double* zntest,
+                     int kernel_id, const double* os, const double* shape, double* Kx, long long ldx, long long stride,
+                     long long n, long long npad, long long mt_rows_pad, long long mt, int dpad, int q, int accumulate,
+                     void* stream) {
     if (!Ztrain || !zntrain || !Ztest || !zntest || !Kx || n <= 0 || npad < n || (npad % 128) || mt <= 0 ||
-        (mt % 128) || mt_rows_pad < mt || ldx < mt || (ldx & 1) || dpad <= 0 || (dpad & 3) || q <= 0 || q > 65535)
+        (mt % 128) || mt_rows_pad < mt || ldx < mt || (ldx & 1) || dpad <= 0 || (dpad & 3) || q <= 0 || q > 65535 ||
+        !shape_arg_ok(kernel_id, shape))
         return PLMC_ERR_BADARG;
     const long long tr = npad / 128, tc = mt / 128;
     if (tr * tc > 2147483647LL) return PLMC_ERR_BADARG;
     const size_t smem = gram_smem(dpad);
     return launch_gram<1>(kernel_id, dim3((unsigned)(tr * tc), 1, q), smem, (cudaStream_t)stream, Ztrain, zntrain,
-                          npad, Ztest, zntest, mt_rows_pad, os, nullptr, Kx, ldx, stride, n, dpad, (int)tc, accumulate);
+                          npad, Ztest, zntest, mt_rows_pad, os, nullptr, Kx, ldx, stride, n, dpad, (int)tc, accumulate,
+                          shape);
 }
 
 int plmc_sweep_debug(int direct) {
@@ -756,22 +821,34 @@ int plmc_sweep_debug(int direct) {
     return PLMC_OK;
 }
 
-long long plmc_grad_ws(long long npad, int d, int q) {
+long long plmc_grad_ws(long long npad, int d, int q) { return plmc_grad_ws2(npad, d, q, PLMC_KERNEL_RBF); }
+
+long long plmc_grad_ws2(long long npad, int d, int q, int kernel_id) {
     if (npad <= 0 || d <= 0 || q <= 0) return 0;
     const long long tm = npad / 128;
     const int dpad = ((d + 3) / 4) * 4;
-    return (long long)q * sweep_ctas(tm * (tm + 1) / 2) * (dpad + 2) * 8;
+    const int nacc = dpad + 2 + (kernel_id == PLMC_KERNEL_RQ ? 1 : 0);
+    return (long long)q * sweep_ctas(tm * (tm + 1) / 2) * nacc * 8;
 }
 
 int plmc_grad_sweep(const double* Kinv, long long ld, long long stride, const double* alpha, long long lda_vec,
                     const double* Z, const double* zn, const double* ell, int kernel_id, const double* os,
                     double* g_ell, double* g_os, double* g_noise, double* partial, long long n, long long npad, int d,
                     int dpad, int q, void* stream) {
+    return plmc_grad_sweep2(Kinv, ld, stride, alpha, lda_vec, Z, zn, ell, kernel_id, os, nullptr, g_ell, g_os, g_noise,
+                            nullptr, partial, n, npad, d, dpad, q, stream);
+}
+
+int plmc_grad_sweep2(const double* Kinv, long long ld, long long stride, const double* alpha, long long lda_vec,
+                     const double* Z, const double* zn, const double* ell, int kernel_id, const double* os,
+                     const double* shape, double* g_ell, double* g_os, double* g_noise, double* g_shape,
+                     double* partial, long long n, long long npad, int d, int dpad, int q, void* stream) {
     if (!Kinv || !alpha || !Z || !zn || !ell || !g_ell || !g_noise || !partial || n <= 0 || npad < n || (npad % 128) ||
         ld < npad || (ld & 1) || d <= 0 || dpad < d || (dpad & 3) || dpad != ((d + 3) / 4) * 4 || q <= 0 ||
-        q > 65535 || lda_vec < n)
+        q > 65535 || lda_vec < n || !shape_arg_ok(kernel_id, shape) || (g_shape && !shape))
         return PLMC_ERR_BADARG;
     cudaStream_t st = (cudaStream_t)stream;
+    const int nacc = dpad + 2 + (kernel_id == PLMC_KERNEL_RQ ? 1 : 0);
     const long long tm = npad / 128;
     const long long ntiles = tm * (tm + 1) / 2;
     const int ctas = sweep_ctas(ntiles);
@@ -783,7 +860,7 @@ int plmc_grad_sweep(const double* Kinv, long long ld, long long stride, const do
     {                                                                                                              \
         cudaFuncSetAttribute(grad_sweep2_kernel<KID, NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2); \
         grad_sweep2_kernel<KID, NB><<<grid2, GR_THREADS, smem2, st>>>(Kinv, ld, stride, alpha, lda_vec, Z, zn, os,   \
-                                                                     partial, n, npad, dpad, ntiles);              \
+                                                                     partial, n, npad, dpad, ntiles, shape);       \
     }
 #define PLMC_SWEEP2_CASE(KID)                                   \
     case KID:                                                   \
@@ -796,18 +873,19 @@ int plmc_grad_sweep(const double* Kinv, long long ld, long long stride, const do
             PLMC_SWEEP2_CASE(1)
             PLMC_SWEEP2_CASE(2)
             PLMC_SWEEP2_CASE(3)
+            PLMC_SWEEP2_CASE(4)
             default: return PLMC_ERR_BADARG;
         }
 #undef PLMC_SWEEP2_CASE
 #undef PLMC_SWEEP2_LAUNCH
         PLMC_CHECK_LAUNCH();
         note_launch(1);
-        grad_reduce_kernel<<<q, 64, 0, st>>>(partial, ctas, d, dpad, ell, g_ell, g_os, g_noise);
+        grad_reduce_kernel<<<q, 64, 0, st>>>(partial, ctas, d, dpad, ell, g_ell, g_os, g_noise, nacc, os, g_shape);
         PLMC_CHECK_LAUNCH();
         note_launch(1);
         return PLMC_OK;
     }
-    const size_t smem = (size_t)(2 * 128 * (dpad + 1) + 256 + 9 * (dpad + 2) + 64 * GR_THREADS) * 8;
+    const size_t smem = (size_t)(2 * 128 * (dpad + 1) + 256 + 9 * nacc + 64 * GR_THREADS) * 8;
     if (smem > 227 * 1024) return PLMC_ERR_BADARG;
     dim3 grid(ctas, 1, q);
 #define PLMC_SWEEP_CASE(KID)                                                                                     \
@@ -815,19 +893,20 @@ int plmc_grad_sweep(const double* Kinv, long long ld, long long stride, const do
         if (smem > 48 * 1024)                                                                                    \
             cudaFuncSetAttribute(grad_sweep_kernel<KID>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
         grad_sweep_kernel<KID><<<grid, GR_THREADS, smem, st>>>(Kinv, ld, stride, alpha, lda_vec, Z, os, partial, n, \
-                                                               npad, dpad, ntiles);                              \
+                                                               npad, dpad, ntiles, shape);                       \
         break;
     switch (kernel_id) {
         PLMC_SWEEP_CASE(0)
         PLMC_SWEEP_CASE(1)
         PLMC_SWEEP_CASE(2)
         PLMC_SWEEP_CASE(3)
+        PLMC_SWEEP_CASE(4)
         default: return PLMC_ERR_BADARG;
     }
 #undef PLMC_SWEEP_CASE
     PLMC_CHECK_LAUNCH();
     note_launch(1);
-    grad_reduce_kernel<<<q, 64, 0, st>>>(partial, ctas, d, dpad, ell, g_ell, g_os, g_noise);
+    grad_reduce_kernel<<<q, 64, 0, st>>>(partial, ctas, d, dpad, ell, g_ell, g_os, g_noise, nacc, os, g_shape);
     PLMC_CHECK_LAUNCH();
     note_launch(1);
     return PLMC_OK;

@@ -245,10 +245,14 @@ class LatentEngine:
     @staticmethod
     def _gram_all(comps, scaled, diag_add, K, n, sl=None):
         """K = sum_g os_g k_g + diag_add I (lower tiles, identity padding); sl restricts to a slice of latents."""
-        for g, ((kid, dims, ell, os_), (Z, zn, _, _)) in enumerate(zip(comps, scaled)):
+        for g, (c, (Z, zn, _, _)) in enumerate(zip(comps, scaled)):
+            kid, dims, ell, os_ = c
+            shape = ops.shape_of(c)
             if sl is not None:
-                Z, zn, os_ = Z[sl], zn[sl], (None if os_ is None else os_[sl])
-            ops.gram(Z, zn, kid, os_, diag_add, K, n, accumulate=(g > 0))
+                Z, zn = Z[sl], zn[sl]
+                os_ = None if os_ is None else os_[sl]
+                shape = None if shape is None else shape[sl]
+            ops.gram(Z, zn, kid, os_, diag_add, K, n, accumulate=(g > 0), shape=shape)
 
     # -- factorisation with gpytorch's psd_safe_cholesky retry semantics ---------
     # The first attempt is launched WITHOUT a host synchronisation: `info` (first bad pivot per latent, like
@@ -264,10 +268,11 @@ class LatentEngine:
         # function of zn, Z, the outputscale and the noise, so the O(qn) inputs are checked instead of the n^2
         # matrix (the integer tensor path would turn a NaN into an arbitrary finite number, not propagate it).
         finite = torch.isfinite(noise).all()
-        for (kid, dims, ell, os_), (Z, zn, _, _) in zip(comps, scaled):
+        for c, (Z, zn, _, _) in zip(comps, scaled):
             finite = finite & torch.isfinite(zn).all()
-            if os_ is not None:
-                finite = finite & torch.isfinite(os_).all()
+            for t in (c[3], ops.shape_of(c)):
+                if t is not None:
+                    finite = finite & torch.isfinite(t).all()
         self.generation += 1
         self._gram_all(comps, scaled, noise, K, n)
         self._mark("gram")
@@ -352,8 +357,9 @@ class LatentEngine:
         np_ = ws["K"].shape[1]
         if need_grad and self.profile is None and 0 < np_ <= self.graph_max_order and X.is_cuda \
                 and not self.capture_mode and not self._force_eager:
-            key = (X.data_ptr(), X._version, tuple(X.shape), q, tuple((kid, tuple(dims), os_ is not None)
-                                                                      for kid, dims, ell, os_ in comps), self._cfg_key)
+            key = (X.data_ptr(), X._version, tuple(X.shape), q,
+                   tuple((c[0], tuple(c[1]), c[3] is not None, ops.shape_of(c) is not None) for c in comps),
+                   self._cfg_key)
             if key in self._graphs:
                 return self._log_prob_and_grads_graphed(ws, key, X, TY, comps, noise, max_tries)
             # the first call with these inputs, kernel structure and arithmetic runs eagerly (lazy library
@@ -396,12 +402,16 @@ class LatentEngine:
         ops.lauum(K, dinv, self.cfg_kinv)
         self._mark("potri")
         g_noise, g_tensors = None, []
-        for (kid, dims, ell, os_), (Z, zn, _, _) in zip(comps, scaled):   # one sweep of K^-1 per additive component
-            g_ell, g_os, g_n = ops.grad_sweep(K, alpha, Z, zn, ell, kid, os_, n)
-            g_noise = g_n if g_noise is None else g_noise
-            g_tensors.append(g_ell)
+        for c, (Z, zn, _, _) in zip(comps, scaled):   # one sweep of K^-1 per additive component
+            kid, dims, ell, os_ = c
+            shape = ops.shape_of(c)
+            g = ops.grad_sweep(K, alpha, Z, zn, ell, kid, os_, n, shape=shape)
+            g_noise = g[2] if g_noise is None else g_noise
+            g_tensors.append(g[0])
             if os_ is not None:
-                g_tensors.append(g_os)
+                g_tensors.append(g[1])
+            if shape is not None:
+                g_tensors.append(g[3])
         self._mark("grad_sweep")
         return lp, (-alpha, g_noise, g_tensors)
 
@@ -428,10 +438,10 @@ class LatentEngine:
         # refresh the static inputs, replay
         st["TY"].copy_(TY)
         st["noise"].copy_(noise)
-        for (kid, dims, ell, os_), (ell_s, os_s) in zip(comps, st["params"]):
-            ell_s.copy_(ell)
-            if os_ is not None:
-                os_s.copy_(os_)
+        for c, static in zip(comps, st["params"]):
+            for src, dst in zip((c[2], c[3], ops.shape_of(c)), static):
+                if src is not None:
+                    dst.copy_(src)
         self.generation += 1
         st["g1"].replay()
         status = self._status_copy(ws["info"])
@@ -447,8 +457,9 @@ class LatentEngine:
 
     def _capture(self, ws, X, TY, comps, noise, n):
         TY_s, noise_s = TY.clone(), noise.clone()
-        params = [(ell.clone(), None if os_ is None else os_.clone()) for kid, dims, ell, os_ in comps]
-        comps_s = [(kid, dims, e, o) for (kid, dims, _, _), (e, o) in zip(comps, params)]
+        # static copies of (ell, os, shape parameter) of every component, refreshed before each replay
+        params = [tuple(None if t is None else t.clone() for t in (c[2], c[3], ops.shape_of(c))) for c in comps]
+        comps_s = [ops.Component(c[0], c[1], e, o, a) for c, (e, o, a) in zip(comps, params)]
         for kid, dims, _, _ in comps_s:
             self._sub_inputs(X, dims)            # column subsets / means are cached outside the graphs
         torch.cuda.synchronize(X.device)
@@ -607,9 +618,10 @@ class LatentEngine:
         zero_padding: the columns of the padding test points are zeroed before the solve, so that V^T V has
         exact zeros outside the ns x ns block."""
         n = st["n"]
-        for g, ((kid, dims, ell, os_), (Z, zn, _, xm)) in enumerate(zip(st["comps"], st["scaled"])):
+        for g, (c, (Z, zn, _, xm)) in enumerate(zip(st["comps"], st["scaled"])):
+            kid, dims, ell, os_ = c
             Zt, znt = ops.scale_inputs(self._component_inputs(xs, dims), xm, ell, mt)
-            ops.cross_gram(Z, zn, Zt, znt, kid, os_, Kx, n, mt, accumulate=(g > 0))
+            ops.cross_gram(Z, zn, Zt, znt, kid, os_, Kx, n, mt, accumulate=(g > 0), shape=ops.shape_of(c))
         lat_mean = ops.latent_mean(Kx, st["alpha"], n, mt)
         if need_v:
             if zero_padding:
@@ -635,9 +647,10 @@ class LatentEngine:
         lat_mean = self._cross_mean_v(st, Xs, V, m, inverted, True, zero_padding=True)[:, :ns].contiguous()
         C = torch.empty((q, m, m), dtype=torch.float64, device=dev)
         zero = torch.zeros(q, dtype=torch.float64, device=dev)
-        for g, ((kid, dims, ell, os_), (_, _, _, xm)) in enumerate(zip(st["comps"], st["scaled"])):
+        for g, (c, (_, _, _, xm)) in enumerate(zip(st["comps"], st["scaled"])):
+            kid, dims, ell, os_ = c
             Zs, zns = ops.scale_inputs(self._component_inputs(Xs, dims), xm, ell, m)
-            ops.gram(Zs, zns, kid, os_, zero, C, ns, accumulate=(g > 0))
+            ops.gram(Zs, zns, kid, os_, zero, C, ns, accumulate=(g > 0), shape=ops.shape_of(c))
         ops.syrk(V, C, -1.0, 1.0, self.cfg_main)
         return lat_mean, C
 

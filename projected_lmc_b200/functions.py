@@ -7,16 +7,20 @@ from . import ops
 
 
 def ops_components(spec, tensors):
-    """[(kernel id, dims, ell, os | None)] from the flat (spec, tensors) form used across the autograd boundary."""
+    """[ops.Component (kernel id, dims, ell, os | None; shape parameter | None)] from the flat (spec, tensors) form
+    used across the autograd boundary.  A spec entry is (kid, dims, has_os) or (kid, dims, has_os, has_shape)."""
     out, i = [], 0
-    for kid, dims, has_os in spec:
+    for kid, dims, has_os, *rest in spec:
         ell = tensors[i]
         i += 1
-        os_ = None
+        os_ = shape = None
         if has_os:
             os_ = tensors[i]
             i += 1
-        out.append((kid, dims, ell, os_))
+        if rest and rest[0]:
+            shape = tensors[i]
+            i += 1
+        out.append(ops.Component(kid, dims, ell, os_, shape))
     return out
 
 
@@ -39,8 +43,8 @@ class ProjectData(torch.autograd.Function):
 class LatentLogProb(torch.autograd.Function):
     """lp_l = log N(TY_l; 0, sum_g o_gl k_gl(X,X) + noise_l I), batched over latents (kernels 2-4).
 
-    ``spec`` = ((kernel id, active dims, has outputscale), ...) describes the additive kernel; ``tensors`` are its
-    parameters in order (ell_0 [q, d_0], os_0 [q] if any, ell_1, ...).  The backward quantities are produced
+    ``spec`` = ((kernel id, active dims, has outputscale, has shape parameter), ...) describes the additive kernel;
+    ``tensors`` are its parameters in order (ell_0 [q, d_0], os_0 [q] if any, alpha_0 [q] if any (RQ), ell_1, ...).  The backward quantities are produced
     eagerly in forward (K -> L -> K^-1 is done in place in one cached workspace, so nothing of size n^2 is saved
     for backward)."""
 

@@ -2,7 +2,7 @@
 
 The Gram matrices themselves are never evaluated in Python: ``kernel_id`` selects
 the fused CUDA epilogue (csrc/gram.cu).  Semantics: gpytorch 1.11 RBFKernel /
-MaternKernel / ScaleKernel as instantiated by handle_covar_ (projected_lmc.py:107-181).
+MaternKernel / RQKernel / ScaleKernel as instantiated by handle_covar_ (projected_lmc.py:107-181).
 """
 from __future__ import annotations
 
@@ -61,6 +61,29 @@ class MaternKernel(Kernel):
     @property
     def kernel_id(self):
         return {2.5: 1, 1.5: 2, 0.5: 3}[self.nu]
+
+
+class RQKernel(Kernel):
+    """gpytorch.kernels.RQKernel: k = (1 + s / (2 alpha))^-alpha on the squared scaled distance s (the RBF input path:
+    centred expansion, clamp_min 0).  ``raw_alpha`` [*batch_shape, 1], initialised to 0, under ``alpha_constraint``
+    (default Positive(), so alpha starts at ln 2); the reference puts no prior on it."""
+    kernel_id = 4
+
+    def __init__(self, alpha_constraint=None, **kwargs):
+        super().__init__(**kwargs)
+        self.register_parameter("raw_alpha", torch.nn.Parameter(torch.zeros(*self.batch_shape, 1)))
+        self.raw_alpha_constraint = alpha_constraint if alpha_constraint is not None else Positive()
+
+    @property
+    def alpha(self) -> torch.Tensor:
+        return self.raw_alpha_constraint.transform(self.raw_alpha)
+
+    @alpha.setter
+    def alpha(self, value):
+        value = torch.as_tensor(value, dtype=self.raw_alpha.dtype, device=self.raw_alpha.device)
+        raw = self.raw_alpha_constraint.inverse_transform(value.expand_as(self.raw_alpha))
+        with torch.no_grad():
+            self.raw_alpha.copy_(raw)
 
 
 class ScaleKernel(torch.nn.Module):

@@ -158,14 +158,16 @@ class ExactGPModel(torch.nn.Module):
         return cm.base_kernel if hasattr(cm, 'base_kernel') else cm
 
     def _kernel_components(self):
-        """[(kernel_id, active dims, lengthscale [q, d_g], outputscale [q] | None)] of the additive kernel."""
+        """[(kernel_id, active dims, lengthscale [q, d_g], outputscale [q] | None)] of the additive kernel
+        (ops.Component: a shape parameter such as RQKernel's alpha [q] rides along as ``.shape_param``)."""
         cm = self._covar()
         out = []
         for ker in (cm.kernels if hasattr(cm, 'kernels') else [cm]):
             base = ker.base_kernel if hasattr(ker, 'base_kernel') else ker
             dims = tuple(range(self.dim)) if base.active_dims is None else tuple(base.active_dims)
-            out.append((base.kernel_id, dims, base.lengthscale.squeeze(-2),
-                        ker.outputscale if hasattr(ker, 'base_kernel') else None))
+            out.append(ops.Component(base.kernel_id, dims, base.lengthscale.squeeze(-2),
+                                     ker.outputscale if hasattr(ker, 'base_kernel') else None,
+                                     base.alpha.squeeze(-1) if hasattr(base, 'raw_alpha') else None))
         return out
 
     def lscales(self, unpacked: bool = True) -> Union[List[Tensor], Tensor]:
@@ -198,7 +200,7 @@ def _resolve_kernel(kernel_type):
     name = getattr(kernel_type, "__name__", str(kernel_type))
     if hasattr(gp.kernels, name):
         return getattr(gp.kernels, name)
-    raise NotImplementedError(f"kernel {name} is not supported on the B200 path (RBFKernel, MaternKernel)")
+    raise NotImplementedError(f"kernel {name} is not supported on the B200 path (RBFKernel, MaternKernel, RQKernel)")
 
 
 class ProjectedGPModel(ExactGPModel):
@@ -362,14 +364,19 @@ class ProjectedGPModel(ExactGPModel):
     # ---- CUDA path -----------------------------------------------------------------
     def _local_components(self, detach=False):
         """(spec, tensors) of the kernel for the latents owned by this process: spec = ((kernel id, dims, has
-        outputscale), ...), tensors = [ell_0, (os_0), ell_1, ...] as contiguous float64."""
+        outputscale, has shape parameter), ...), tensors = [ell_0, (os_0), (alpha_0), ell_1, ...] as contiguous
+        float64."""
         lo, hi = self._latent_range
         spec, tensors = [], []
-        for kid, dims, ell, os_ in self._kernel_components():
-            spec.append((kid, dims, os_ is not None))
+        for comp in self._kernel_components():
+            kid, dims, ell, os_ = comp
+            shape = ops.shape_of(comp)
+            spec.append((kid, dims, os_ is not None, shape is not None))
             tensors.append(_as_f64(ell)[lo:hi])
             if os_ is not None:
                 tensors.append(_as_f64(os_)[lo:hi])
+            if shape is not None:
+                tensors.append(_as_f64(shape)[lo:hi])
         if detach:
             tensors = [t.detach().contiguous() for t in tensors]
         return tuple(spec), tensors
@@ -455,12 +462,21 @@ class ProjectedGPModel(ExactGPModel):
             m, v = self._predict_latents(st, xs)
         return LatentPosterior(m.to(x.dtype), v.to(x.dtype), _JointPosterior(self, xs, x.dtype))
 
+    def _full_components(self):
+        """The kernel components of all latents as contiguous float64 (no autograd)."""
+        def f64(t):
+            return None if t is None else _as_f64(t).contiguous()
+        out = []
+        for c in self._kernel_components():
+            kid, dims, ell, os_ = c
+            out.append(ops.Component(kid, dims, f64(ell), f64(os_), f64(ops.shape_of(c))))
+        return out
+
     def kernel_cond(self):
         """Condition numbers of the noisy latent train covariances K_l + s_l I (dense SVD: small n)."""
         with torch.no_grad():
             X = _as_f64(self.train_inputs[0])
-            comps = [(kid, dims, _as_f64(ell).contiguous(), None if os_ is None else _as_f64(os_).contiguous())
-                     for kid, dims, ell, os_ in self._kernel_components()]
+            comps = self._full_components()
             K = self._engine.dense_gram(X, comps, _as_f64(self.projected_noise()).contiguous())
             return torch.linalg.cond(K)
 
@@ -469,8 +485,7 @@ class ProjectedGPModel(ExactGPModel):
         both n_points x n_latents (by-product of K^-1 and alpha)."""
         with torch.no_grad():
             X = _as_f64(self.train_inputs[0])
-            comps = [(kid, dims, _as_f64(ell).contiguous(), None if os_ is None else _as_f64(os_).contiguous())
-                     for kid, dims, ell, os_ in self._kernel_components()]
+            comps = self._full_components()
             TY = _as_f64(self.project_data(self.train_y)).contiguous()
             s2, r = self._engine.loo(X, TY, comps, _as_f64(self.projected_noise()).contiguous())
         dt = self.train_y.dtype

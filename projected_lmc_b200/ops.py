@@ -14,7 +14,26 @@ from . import _cabi
 from ._cabi import (GEMM_FLAG_SINGLE_CTA, GEMM_FP64, GEMM_INT8_DIGITS, GEMM_INT8_RNS, GemmCfg, PlmcError, check, lib,
                     npad, ptr, stream)
 
-KERNEL_IDS = {"rbf": 0, "matern52": 1, "matern32": 2, "matern12": 3}
+KERNEL_IDS = {"rbf": 0, "matern52": 1, "matern32": 2, "matern12": 3, "rq": 4}
+KERNEL_RQ = 4
+# kernels with a shape parameter (one value per latent): the ...2 entry points carry it
+SHAPED_KERNELS = frozenset({KERNEL_RQ})
+
+
+class Component(tuple):
+    """One additive kernel component, (kernel id, dims, ell [q, d_g], os [q] | None), with the kernel's shape
+    parameter [q] (RQ: alpha) as ``.shape_param``.  It unpacks as the plain 4-tuple of the kernels without one,
+    which callers may keep using."""
+
+    def __new__(cls, kid, dims, ell, os_, shape_param=None):
+        self = super().__new__(cls, (kid, dims, ell, os_))
+        self.shape_param = shape_param
+        return self
+
+
+def shape_of(comp):
+    """The shape parameter of a component (None for a plain 4-tuple or a kernel without one)."""
+    return getattr(comp, "shape_param", None)
 
 # layout codes of plmc_gemm: bit1 -> A(m,k) m-contiguous, bit0 -> B(k,n) n-contiguous
 A_KC_B_KC, A_KC_B_NC, A_MC_B_KC, A_MC_B_NC = 0, 1, 2, 3
@@ -202,62 +221,78 @@ def scale_inputs(X, xmean, ell, rows_pad):
     return Z, zn
 
 
+def _check_shape(kernel_id, shape):
+    if (kernel_id in SHAPED_KERNELS) != (shape is not None):
+        raise PlmcError(f"kernel {kernel_id}: a shape parameter is required by the rational quadratic kernel and "
+                        "refused by the others")
+
+
 @_on_device
-def gram(Z, zn, kernel_id, os_, diag_add, K, n, accumulate=False):
+def gram(Z, zn, kernel_id, os_, diag_add, K, n, accumulate=False, *, shape=None):
+    """shape: the kernel's shape parameter [q] (RQ alpha), None for kernels without one."""
+    _check_shape(kernel_id, shape)
     q, np_, dp = Z.shape
     check(
-        lib().plmc_gram(ptr(Z), ptr(zn), kernel_id, ptr(os_), ptr(diag_add), ptr(K), K.stride(1), K.stride(0), n, np_,
-                        dp, q, int(accumulate), stream()),
+        lib().plmc_gram2(ptr(Z), ptr(zn), kernel_id, ptr(os_), ptr(shape), ptr(diag_add), ptr(K), K.stride(1),
+                         K.stride(0), n, np_, dp, q, int(accumulate), stream()),
         "gram",
     )
 
 
 @_on_device
-def cross_gram(Ztr, zntr, Zte, znte, kernel_id, os_, Kx, n, mt, accumulate=False):
+def cross_gram(Ztr, zntr, Zte, znte, kernel_id, os_, Kx, n, mt, accumulate=False, *, shape=None):
+    _check_shape(kernel_id, shape)
     q, np_, dp = Ztr.shape
     check(
-        lib().plmc_cross_gram(ptr(Ztr), ptr(zntr), ptr(Zte), ptr(znte), kernel_id, ptr(os_), ptr(Kx), Kx.stride(1),
-                              Kx.stride(0), n, np_, Zte.shape[1], mt, dp, q, int(accumulate), stream()),
+        lib().plmc_cross_gram2(ptr(Ztr), ptr(zntr), ptr(Zte), ptr(znte), kernel_id, ptr(os_), ptr(shape), ptr(Kx),
+                               Kx.stride(1), Kx.stride(0), n, np_, Zte.shape[1], mt, dp, q, int(accumulate), stream()),
         "cross_gram",
     )
 
 
 @_on_device
-def cross_gram_bwd(Zr, Zc, G, kernel_id, os_, ell, nr, nc):
+def cross_gram_bwd(Zr, Zc, G, kernel_id, os_, ell, nr, nc, *, shape=None):
     """Adjoint of K[l,i,j] = os[l] k(|zr_i - zc_j|^2) for the cotangent G [q, nr, >=nc]:
-    (g_ell [q, d], g_os [q], g_rows [nr, d] summed over latents, w.r.t. the unscaled row points)."""
+    (g_ell [q, d], g_os [q], g_rows [nr, d] summed over latents, w.r.t. the unscaled row points), and g_shape [q]
+    appended when the kernel has a shape parameter."""
+    _check_shape(kernel_id, shape)
     q, rpr, dp = Zr.shape
     rpc = Zc.shape[1]
     d = ell.shape[1]
     dev = G.device
-    ws = torch.empty((lib().plmc_cross_gram_bwd_ws(nr, nc, d, q) // 8,), dtype=torch.float64, device=dev)
+    ws = torch.empty((lib().plmc_cross_gram_bwd_ws2(nr, nc, d, q, kernel_id) // 8,), dtype=torch.float64, device=dev)
     g_ell = torch.empty((q, d), dtype=torch.float64, device=dev)
     g_os = torch.empty((q,), dtype=torch.float64, device=dev)
     g_rows = torch.empty((nr, d), dtype=torch.float64, device=dev)
+    g_shape = None if shape is None else torch.empty((q,), dtype=torch.float64, device=dev)
     check(
-        lib().plmc_cross_gram_bwd(ptr(Zr), rpr, ptr(Zc), rpc, ptr(G), G.stride(1), G.stride(0), kernel_id, ptr(os_),
-                                  ptr(ell), ptr(g_ell), ptr(g_os), ptr(g_rows), ptr(ws), nr, nc, d, dp, q, stream()),
+        lib().plmc_cross_gram_bwd2(ptr(Zr), rpr, ptr(Zc), rpc, ptr(G), G.stride(1), G.stride(0), kernel_id, ptr(os_),
+                                   ptr(shape), ptr(ell), ptr(g_ell), ptr(g_os), ptr(g_shape), ptr(g_rows), ptr(ws), nr,
+                                   nc, d, dp, q, stream()),
         "cross_gram_bwd",
     )
-    return g_ell, g_os, g_rows
+    return (g_ell, g_os, g_rows) if shape is None else (g_ell, g_os, g_rows, g_shape)
 
 
 @_on_device
-def grad_sweep(Kinv, alpha, Z, zn, ell, kernel_id, os_, n):
+def grad_sweep(Kinv, alpha, Z, zn, ell, kernel_id, os_, n, *, shape=None):
+    """(g_ell, g_os, g_noise), and g_shape [q] appended when the kernel has a shape parameter."""
+    _check_shape(kernel_id, shape)
     q, np_, dp = Z.shape
     d = ell.shape[1]
     dev = Kinv.device
-    ws = torch.empty((lib().plmc_grad_ws(np_, d, q) // 8,), dtype=torch.float64, device=dev)
+    ws = torch.empty((lib().plmc_grad_ws2(np_, d, q, kernel_id) // 8,), dtype=torch.float64, device=dev)
     g_ell = torch.empty((q, d), dtype=torch.float64, device=dev)
     g_os = torch.empty((q,), dtype=torch.float64, device=dev)
     g_noise = torch.empty((q,), dtype=torch.float64, device=dev)
+    g_shape = None if shape is None else torch.empty((q,), dtype=torch.float64, device=dev)
     check(
-        lib().plmc_grad_sweep(ptr(Kinv), Kinv.stride(1), Kinv.stride(0), ptr(alpha), alpha.stride(0), ptr(Z), ptr(zn),
-                              ptr(ell), kernel_id, ptr(os_), ptr(g_ell), ptr(g_os), ptr(g_noise), ptr(ws), n, np_, d,
-                              dp, q, stream()),
+        lib().plmc_grad_sweep2(ptr(Kinv), Kinv.stride(1), Kinv.stride(0), ptr(alpha), alpha.stride(0), ptr(Z), ptr(zn),
+                               ptr(ell), kernel_id, ptr(os_), ptr(shape), ptr(g_ell), ptr(g_os), ptr(g_noise),
+                               ptr(g_shape), ptr(ws), n, np_, d, dp, q, stream()),
         "grad_sweep",
     )
-    return g_ell, g_os, g_noise
+    return (g_ell, g_os, g_noise) if shape is None else (g_ell, g_os, g_noise, g_shape)
 
 
 @_on_device

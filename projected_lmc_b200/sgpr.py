@@ -24,33 +24,40 @@ from .gp import settings
 
 class CrossGram(torch.autograd.Function):
     """K[l, i, j] = os_l k(|(u_i - x_j) / ell_l|^2): rows = points U [m, d] (differentiable), columns = data X [n, d].
-    ``symmetric``: X is U itself (K_uu); the adjoint then accounts for both roles of U."""
+    ``symmetric``: X is U itself (K_uu); the adjoint then accounts for both roles of U.  ``shape``: the kernel's
+    shape parameter [q] (RQ alpha), None for kernels without one."""
 
     @staticmethod
-    def forward(ctx, U, X, xmean, kid, ell, os_, symmetric):
+    def forward(ctx, U, X, xmean, kid, ell, os_, symmetric, shape=None):
         m, n = U.shape[0], X.shape[0]
         Ud, ed = U.detach().contiguous(), ell.detach().contiguous()
         od = None if os_ is None else os_.detach().contiguous()
+        ad = None if shape is None else shape.detach().contiguous()
         mp, np_ = _npad(m), _npad(n)
         Zr, znr = ops.scale_inputs(Ud, xmean, ed, mp)
         Zc, znc = (Zr, znr) if symmetric else ops.scale_inputs(X.detach().contiguous(), xmean, ed, np_)
         Kx = torch.empty((ed.shape[0], mp, np_), dtype=torch.float64, device=U.device)
-        ops.cross_gram(Zr, znr, Zc, znc, kid, od, Kx, m, np_)
-        ctx.save_for_backward(Zr, Zc, ed, od if od is not None else torch.empty(0, device=U.device))
-        ctx.meta = (kid, m, n, od is not None, symmetric)
+        ops.cross_gram(Zr, znr, Zc, znc, kid, od, Kx, m, np_, shape=ad)
+        empty = torch.empty(0, device=U.device)
+        ctx.save_for_backward(Zr, Zc, ed, od if od is not None else empty, ad if ad is not None else empty)
+        ctx.meta = (kid, m, n, od is not None, symmetric, ad is not None)
         return Kx[:, :m, :n]
 
     @staticmethod
     def backward(ctx, G):
-        Zr, Zc, ell, os_ = ctx.saved_tensors
-        kid, m, n, has_os, symmetric = ctx.meta
+        Zr, Zc, ell, os_, shape = ctx.saved_tensors
+        kid, m, n, has_os, symmetric, has_shape = ctx.meta
         G = G.contiguous()
         if symmetric:
             G = G + G.transpose(1, 2)
-        g_ell, g_os, g_rows = ops.cross_gram_bwd(Zr, Zc, G, kid, os_ if has_os else None, ell, m, n)
-        if symmetric:   # each unordered pair was counted twice in the lengthscale / outputscale sums
+        g = ops.cross_gram_bwd(Zr, Zc, G, kid, os_ if has_os else None, ell, m, n,
+                               shape=shape if has_shape else None)
+        g_ell, g_os, g_rows = g[0], g[1], g[2]
+        g_shape = g[3] if has_shape else None
+        if symmetric:   # each unordered pair was counted twice in the lengthscale / outputscale / shape sums
             g_ell, g_os = 0.5 * g_ell, 0.5 * g_os
-        return g_rows, None, None, None, g_ell, (g_os if has_os else None), None
+            g_shape = None if g_shape is None else 0.5 * g_shape
+        return g_rows, None, None, None, g_ell, (g_os if has_os else None), None, g_shape
 
 
 def _chol_safe(A: torch.Tensor, max_tries: int):
@@ -75,11 +82,12 @@ def _chol_safe(A: torch.Tensor, max_tries: int):
 def _blocks(engine, X, U, comps):
     """(K_uu [q, m, m], K_uf [q, m, n], prior variance [q]) of the additive kernel."""
     Kuu = Kuf = kss = None
-    for kid, dims, ell, os_ in comps:
+    for c in comps:
+        kid, dims, ell, os_ = c
         Xg, xm = engine._sub_inputs(X, dims)
         Ug = U if len(dims) == U.shape[1] and tuple(dims) == tuple(range(U.shape[1])) else U[:, list(dims)]
-        a = CrossGram.apply(Ug, Ug, xm, kid, ell, os_, True)
-        b = CrossGram.apply(Ug, Xg, xm, kid, ell, os_, False)
+        a = CrossGram.apply(Ug, Ug, xm, kid, ell, os_, True, ops.shape_of(c))
+        b = CrossGram.apply(Ug, Xg, xm, kid, ell, os_, False, ops.shape_of(c))
         v = torch.ones(ell.shape[0], dtype=torch.float64, device=X.device) if os_ is None else os_
         Kuu, Kuf, kss = (a, b, v) if Kuu is None else (Kuu + a, Kuf + b, kss + v)
     return Kuu, Kuf, kss
@@ -130,11 +138,12 @@ def predict_latents(engine, st, X, Xs, tile=65536):
     for s0 in range(0, ns, tile):
         xs = Xs[s0:s0 + tile]
         Kus = None
-        for kid, dims, ell, os_ in st["comps"]:
+        for c in st["comps"]:
+            kid, dims, ell, os_ = c
             _, xm = engine._sub_inputs(X, dims)
             full = len(dims) == U.shape[1] and tuple(dims) == tuple(range(U.shape[1]))
             Ug, xg = (U, xs) if full else (U[:, list(dims)], xs[:, list(dims)].contiguous())
-            b = CrossGram.apply(Ug, xg, xm, kid, ell, os_, False)
+            b = CrossGram.apply(Ug, xg, xm, kid, ell, os_, False, ops.shape_of(c))
             Kus = b if Kus is None else Kus + b
         As = torch.linalg.solve_triangular(st["Luu"], Kus, upper=False)                      # [q, m, t]
         mean[:, s0:s0 + tile] = (As * st["w"]).sum(1)
