@@ -287,7 +287,7 @@ def test_gram_and_cross_gram_vs_oracle(kind, kid, n, d, with_os):
     assert Kx[:, n:, :].abs().max().item() == 0.0 if np_ > n else True
 
 
-@pytest.mark.parametrize("kind,kid", [("rbf", 0), ("matern52", 1), ("matern32", 2)])
+@pytest.mark.parametrize("kind,kid", [("rbf", 0), ("matern52", 1), ("matern32", 2), ("matern12", 3)])
 @pytest.mark.parametrize("n,d,with_os", [(100, 1, False), (300, 6, True), (257, 21, False), (640, 12, True),
                                          (200, 24, False), (150, 30, True)])
 def test_gradient_sweep_both_kernels_vs_autograd(kind, kid, n, d, with_os):
