@@ -256,6 +256,29 @@ int plmc_mix_tasks(const double* lat_mean, const double* lat_var, long long ldm,
                    const double* var_add, double* mean, double* var, long long mt, int p, int q, int accumulate,
                    void* stream);
 
+/* ---- gradients of the predictive means / variances w.r.t. the test inputs: autograd of the eval branch of
+ * ProjectedGPModel.__call__ (projected_lmc.py:1121-1155) through gpytorch exact_prediction.
+ * plmc_mix_tasks_bwd is the transpose of plmc_mix_tasks: g_lat_mean[l,j] = sum_t g_mean[j,t] H[l,t] and
+ * g_lat_var[l,j] = sum_t g_var[j,t] H[l,t]^2 for cotangents [mt, p] (either may be NULL, together with its output;
+ * not both); outputs [q, ldm].                                                                                      */
+int plmc_mix_tasks_bwd(const double* g_mean, const double* g_var, const double* H, double* g_lat_mean,
+                       double* g_lat_var, long long ldm, long long mt, int p, int q, void* stream);
+/* One additive component's share of d/dx* of sum_j (g_mean[l,j] mu_l(j) + g_var[l,j] v_l(j)), summed over latents:
+ *   g_x[j, k] = sum_l (2/ell[l,k]) sum_i A[i,j] (z*_jk - z_ik),  A[i,j] = w[i,j] os[l] k'(s_ij),
+ *   w[i,j] = g_mean[l,j] alpha[l,i] - 2 g_var[l,j] beta[l,i,j],  beta = K^-1 K* [q, npad, ldb] (batch stride strideb).
+ * Ztrain / zntrain [q, npad, dpad] / [q, npad] and Ztest / zntest [q, rows_pad_test, dpad] from plmc_scale_inputs
+ * (rows_pad_test >= ns rounded up to 64); alpha [q, lda]; g_mean / g_var [q, ldg]; g_x [ns, ldx] (the unscaled inputs
+ * of this component).  g_var and beta come together: without them nothing of size n x ns is read.  Test columns
+ * >= ns do not affect the result, whatever the padding of beta holds.  dpad <= 48; shape as plmc_cross_gram2.
+ * partial: plmc_cross_grad_ws(npad, ns, d, q) bytes.  Deterministic (fixed-order reductions, no atomics).         */
+long long plmc_cross_grad_ws(long long npad, long long ns, int d, int q);
+int plmc_cross_grad(const double* Ztrain, const double* zntrain, long long npad, const double* Ztest,
+                    const double* zntest, long long rows_pad_test, int kernel_id, const double* os,
+                    const double* shape, const double* ell, const double* alpha, long long lda, const double* g_mean,
+                    const double* g_var, long long ldg, const double* beta, long long ldb, long long strideb,
+                    double* g_x, long long ldx, double* partial, long long n, long long ns, int d, int dpad, int q,
+                    void* stream);
+
 /* ---- joint predictive covariance and posterior draws (the full MultitaskMultivariateNormal of the eval branch,
  * projected_lmc.py:1149-1155: covariance sum_l C_l (x) h_l h_l^T + eps I, + I (x) F F^T after full_likelihood).
  * Latent posterior covariance C_l = K**_l - V_l^T V_l:  K**_l from plmc_gram on the scaled test points (diag_add 0),

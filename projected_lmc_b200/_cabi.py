@@ -75,6 +75,9 @@ _SIGNATURES = {
     "plmc_latent_mean": [P, LL, LL, P, LL, P, LL, LL, LL, I, P],
     "plmc_latent_var": [P, LL, LL, P, P, LL, LL, LL, I, P],
     "plmc_mix_tasks": [P, P, LL, P, P, P, P, LL, I, I, I, P],
+    "plmc_mix_tasks_bwd": [P, P, P, P, P, LL, LL, I, I, P],
+    "plmc_cross_grad_ws": [LL, LL, I, I],
+    "plmc_cross_grad": [P, P, LL, P, P, LL, I, P, P, P, P, LL, P, P, LL, P, LL, LL, P, LL, P, LL, LL, I, I, I, P],
     "plmc_syrk_batched": [P, LL, LL, P, LL, LL, LL, LL, D, D, I, CFG, P],
     "plmc_task_covariance": [P, LL, LL, P, P, P, LL, LL, I, I, I, P],
     "plmc_mix_samples": [P, P, LL, LL, P, P, P, P, LL, LL, I, I, P],
@@ -92,7 +95,8 @@ _SIGNATURES = {
     "plmc_peak_mixed": [I, I, LL, LL, P, P],
 }
 _RET_LL = {"plmc_npad", "plmc_dinv_bytes", "plmc_project_bwd_ws", "plmc_grad_ws", "plmc_ozaki_ws_bytes",
-           "plmc_rns_ws_bytes", "plmc_cross_gram_bwd_ws", "plmc_grad_ws2", "plmc_cross_gram_bwd_ws2"}
+           "plmc_rns_ws_bytes", "plmc_cross_gram_bwd_ws", "plmc_grad_ws2", "plmc_cross_gram_bwd_ws2",
+           "plmc_cross_grad_ws"}
 
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

@@ -606,6 +606,59 @@ class LatentEngine:
                 lat_var[:, s0:s0 + cnt] = ops.latent_var(Kx, st["prior_var"], mt)[:, :cnt]
         return lat_mean, lat_var
 
+    def predict_latents_grad(self, st, Xs, g_mean=None, g_var=None, tile=None):
+        """Gradient w.r.t. the test points Xs [n*, d] of sum_lj g_mean[l,j] mu_l(j) + g_var[l,j] v_l(j) for latent
+        cotangents [q, n*] (either may be None): [n*, d].  Nothing is kept from the forward: each tile rebuilds K*
+        and, with variance cotangents only, beta = K^-1 K* = L^-T (L^-1 K*) in place (trmm by the explicit inverse
+        once the state is inverted, else trsm), so the memory is that of one prediction tile."""
+        q, np_ = self._check_state(st, Xs.device)
+        ns, d = Xs.shape
+        dev = Xs.device
+        out = torch.zeros((ns, d), dtype=torch.float64, device=dev)
+        if g_mean is None and g_var is None:
+            return out
+        g_mean = None if g_mean is None else g_mean.contiguous()
+        g_var = None if g_var is None else g_var.contiguous()
+        mt_full = tile or self.tile_points(q, np_, device=dev)
+        inverted = bool(st.get("inverted"))
+        n = st["n"]
+        Kx = None
+        for s0 in range(0, ns, mt_full):
+            cnt = min(mt_full, ns - s0)
+            mt = _npad(cnt)
+            if Kx is None or Kx.shape[2] != mt:
+                Kx = None
+                Kx = torch.empty((q, np_, mt), dtype=torch.float64, device=dev)
+            xs = Xs[s0:s0 + cnt]
+            scaled_t = []
+            for g, (c, (_, _, _, xm)) in enumerate(zip(st["comps"], st["scaled"])):
+                kid, dims, ell, os_ = c
+                Zt, znt = ops.scale_inputs(self._component_inputs(xs, dims), xm, ell, mt)
+                scaled_t.append((Zt, znt))
+                if g_var is not None:
+                    ops.cross_gram(st["scaled"][g][0], st["scaled"][g][1], Zt, znt, kid, os_, Kx, n, mt,
+                                   accumulate=(g > 0), shape=ops.shape_of(c))
+            beta = None
+            if g_var is not None:
+                if inverted:
+                    ops.trmm(2, st["L"], st["dinv"], Kx, 1.0, self.cfg_main)
+                    ops.trmm(3, st["L"], st["dinv"], Kx, 1.0, self.cfg_main)
+                else:
+                    ops.trsm(2, st["L"], st["dinv"], Kx, 1.0, self.cfg_main)
+                    ops.trsm(3, st["L"], st["dinv"], Kx, 1.0, self.cfg_main)
+                beta = Kx
+            gm = None if g_mean is None else g_mean[:, s0:s0 + cnt]
+            gv = None if g_var is None else g_var[:, s0:s0 + cnt]
+            for c, (Z, zn, _, _), (Zt, znt) in zip(st["comps"], st["scaled"], scaled_t):
+                kid, dims, ell, os_ = c
+                gx = ops.cross_grad(Z, zn, Zt, znt, kid, os_, ell, st["alpha"], n, cnt, gm, gv, beta,
+                                    shape=ops.shape_of(c))
+                if tuple(dims) == tuple(range(d)):
+                    out[s0:s0 + cnt] += gx
+                else:
+                    out[s0:s0 + cnt].index_add_(1, torch.as_tensor(list(dims), device=dev), gx)
+        return out
+
     @staticmethod
     def _component_inputs(xs, dims):
         if len(dims) == xs.shape[1] and tuple(dims) == tuple(range(xs.shape[1])):

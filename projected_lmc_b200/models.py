@@ -17,6 +17,7 @@ from typing import List, Optional, Union
 import numpy as np
 import torch
 from torch import Tensor
+from torch.autograd.function import once_differentiable
 
 from . import gp, ops
 from .engine import LatentEngine
@@ -456,11 +457,21 @@ class ProjectedGPModel(ExactGPModel):
         if self.training:
             self._check_train_inputs(x)
             return self.forward(x)
+        if self._input_grad(x):
+            xs = _as_f64(x if x.dim() > 1 else x.unsqueeze(-1)).contiguous()
+            m, v = _LatentPrediction.apply(self, xs, False)
+            return LatentPosterior(m.to(x.dtype), v.to(x.dtype), _JointPosterior(self, xs.detach(), x.dtype))
         with torch.no_grad():
             st = self._prediction_state()
             xs = _as_f64(x if x.dim() > 1 else x.unsqueeze(-1)).contiguous()
             m, v = self._predict_latents(st, xs)
         return LatentPosterior(m.to(x.dtype), v.to(x.dtype), _JointPosterior(self, xs, x.dtype))
+
+    def _input_grad(self, x: Tensor) -> bool:
+        """Eval-mode predictions are differentiable w.r.t. the test inputs when grad is enabled and x requires it
+        (not for latent-sharded models, whose outputs stay detached)."""
+        return torch.is_grad_enabled() and x.requires_grad and self._dist_group is None and \
+            self._latent_range == (0, self.n_latents)
 
     def _full_components(self):
         """The kernel components of all latents as contiguous float64 (no autograd)."""
@@ -497,6 +508,8 @@ class ProjectedGPModel(ExactGPModel):
         if self.training:
             self._check_train_inputs(x)
             return self.forward(x)
+        if self._input_grad(x):
+            return self._differentiable_call(x)
         with torch.no_grad():
             st = self._prediction_state()
             xs = _as_f64(x if x.dim() > 1 else x.unsqueeze(-1)).contiguous()
@@ -528,6 +541,100 @@ class ProjectedGPModel(ExactGPModel):
             joint.task_mean = mean
             task_noise = float(self.eps) * torch.eye(self.n_tasks, dtype=torch.float64, device=xs.device)
         return gp.distributions.MultitaskMultivariateNormal(mean.to(x.dtype), var.to(x.dtype), joint, task_noise)
+
+    def _differentiable_call(self, x: Tensor):
+        """The eval branch of __call__ with .mean / .variance differentiable w.r.t. x (same values, bit for bit).
+        Model parameters receive no gradient through predictions; the joint quantities (covariance_matrix, rsample,
+        log_prob) stay detached."""
+        xs = _as_f64(x if x.dim() > 1 else x.unsqueeze(-1)).contiguous()
+        joint = _JointPosterior(self, xs.detach(), x.dtype)
+        bad_rows = ~torch.isfinite(xs.detach()).all(dim=1)
+        lat_mean, lat_var = _LatentPrediction.apply(self, xs, True)
+        with torch.no_grad():
+            Ht = _as_f64(self.lmc_coefficients()).contiguous()
+            var_add = torch.full((self.n_tasks,), float(self.eps), dtype=torch.float64, device=xs.device)
+        mean, var = _MixTasks.apply(lat_mean, lat_var, Ht, var_add)
+        if bool(bad_rows.any()):
+            mean = mean.masked_fill(bad_rows[:, None], float("nan"))
+            var = var.masked_fill(bad_rows[:, None], float("nan"))
+        joint.task_mean = mean.detach()
+        task_noise = float(self.eps) * torch.eye(self.n_tasks, dtype=torch.float64, device=xs.device)
+        return gp.distributions.MultitaskMultivariateNormal(mean.to(x.dtype), var.to(x.dtype), joint, task_noise)
+
+
+class _LatentPrediction(torch.autograd.Function):
+    """Latent posterior means / variances [q, n*] at the float64 test points xs [n*, d] of an eval-mode model, with
+    their gradient w.r.t. xs.  The forward is the model's no-grad prediction (``zero_bad``: non-finite rows are
+    predicted at 0, as ProjectedGPModel.__call__ does).  The backward keeps nothing of size n x n* from the forward:
+    the exact model recomputes each tile in LatentEngine.predict_latents_grad, the inducing-point model runs torch
+    autograd through its cross block with the test points as rows.  A parameter or train_y changed since the forward
+    is an error; a rewritten engine workspace (compute_loo, a training step) is re-factorised.  Rows of non-finite
+    test points get NaN gradients.  Not twice differentiable."""
+
+    @staticmethod
+    def forward(ctx, model, xs, zero_bad):
+        xin = xs
+        bad_rows = ~torch.isfinite(xs).all(dim=1)
+        if zero_bad and bool(bad_rows.any()):
+            xin = xs.clone()
+            xin[bad_rows] = 0.0
+        st = model._prediction_state()
+        m, v = model._predict_latents(st, xin)
+        ctx.model, ctx.key = model, model._parameter_key()
+        ctx.save_for_backward(xs)
+        ctx.set_materialize_grads(False)
+        return m, v
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_mean, g_var):
+        model = ctx.model
+        (xs,) = ctx.saved_tensors
+        if g_mean is None and g_var is None:
+            return None, None, None
+        if model._parameter_key() != ctx.key:
+            raise RuntimeError("the model's parameters or train_y changed after this prediction was made; "
+                               "call the model again before backpropagating to the test inputs")
+        bad_rows = ~torch.isfinite(xs).all(dim=1)
+        has_bad = bool(bad_rows.any())
+        x0 = xs.masked_fill(bad_rows[:, None], 0.0) if has_bad else xs
+        st = model._prediction_state()
+        if model._inducing() is not None:
+            from . import sgpr
+            with torch.enable_grad():
+                xr = x0.detach().requires_grad_(True)
+                m, v = sgpr.predict_latents(model._engine, st, _as_f64(model.train_inputs[0]), xr, test_rows=True)
+                outs = [(o, g) for o, g in ((m, g_mean), (v, g_var)) if g is not None]
+                (g,) = torch.autograd.grad([o for o, _ in outs], (xr,), [g for _, g in outs])
+        else:
+            g = model._engine.predict_latents_grad(st, x0, g_mean, g_var)
+        if has_bad:
+            g[bad_rows] = float("nan")
+        return None, g, None
+
+
+class _MixTasks(torch.autograd.Function):
+    """Task-level means / marginal variances [n*, p] from the latent ones (ops.mix_tasks), differentiable w.r.t. the
+    latent means and variances (ops.mix_tasks_bwd); H and var_add receive no gradient."""
+
+    @staticmethod
+    def forward(ctx, lat_mean, lat_var, H, var_add):
+        ns = lat_mean.shape[1]
+        mean = torch.empty((ns, H.shape[1]), dtype=torch.float64, device=lat_mean.device)
+        var = torch.empty_like(mean)
+        ops.mix_tasks(lat_mean, lat_var, H, var_add, mean, var, ns)
+        ctx.H = H
+        ctx.set_materialize_grads(False)
+        return mean, var
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g_mean, g_var):
+        if g_mean is None and g_var is None:
+            return None, None, None, None
+        g_lm, g_lv = ops.mix_tasks_bwd(ctx.H, None if g_mean is None else g_mean.contiguous(),
+                                       None if g_var is None else g_var.contiguous())
+        return g_lm, g_lv, None, None
 
 
 class _StoredLoss:

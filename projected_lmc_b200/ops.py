@@ -321,6 +321,46 @@ def mix_tasks(lat_mean, lat_var, H, var_add, mean, var, mt, accumulate=False):
 
 
 @_on_device
+def mix_tasks_bwd(H, g_mean=None, g_var=None, mt=None):
+    """Transpose of mix_tasks for the cotangents g_mean / g_var [mt, p] (either may be None):
+    (g_lat_mean [q, mt] | None, g_lat_var [q, mt] | None)."""
+    q, p = H.shape
+    ref = g_mean if g_mean is not None else g_var
+    mt = ref.shape[0] if mt is None else mt
+    g_lm = None if g_mean is None else torch.empty((q, mt), dtype=torch.float64, device=H.device)
+    g_lv = None if g_var is None else torch.empty((q, mt), dtype=torch.float64, device=H.device)
+    check(lib().plmc_mix_tasks_bwd(ptr(g_mean), ptr(g_var), ptr(H), ptr(g_lm), ptr(g_lv), mt, mt, p, q, stream()),
+          "mix_tasks_bwd")
+    return g_lm, g_lv
+
+
+@_on_device
+def cross_grad(Ztr, zntr, Zte, znte, kernel_id, os_, ell, alpha, n, ns, g_mean=None, g_var=None, beta=None, *,
+               shape=None):
+    """One component's share of the gradient w.r.t. the (unscaled) test points [ns, d] of
+    sum_lj g_mean[l,j] mu_l(j) + g_var[l,j] v_l(j), summed over latents.  g_mean / g_var [q, >=ns] (views with unit
+    column stride); beta = K^-1 K* [q, npad, >=ns], required with g_var and only then."""
+    _check_shape(kernel_id, shape)
+    q, np_, dp = Ztr.shape
+    d = ell.shape[1]
+    dev = Ztr.device
+    ws = torch.empty((lib().plmc_cross_grad_ws(np_, ns, d, q) // 8,), dtype=torch.float64, device=dev)
+    g_x = torch.empty((ns, d), dtype=torch.float64, device=dev)
+    if g_mean is not None and g_var is not None and g_mean.stride(0) != g_var.stride(0):
+        g_mean, g_var = g_mean.contiguous(), g_var.contiguous()      # the C entry point takes one leading dimension
+    ref = g_mean if g_mean is not None else g_var
+    ldg = 0 if ref is None else ref.stride(0)
+    ldb, sb = (0, 0) if beta is None else (beta.stride(1), beta.stride(0))
+    check(
+        lib().plmc_cross_grad(ptr(Ztr), ptr(zntr), np_, ptr(Zte), ptr(znte), Zte.shape[1], kernel_id, ptr(os_),
+                              ptr(shape), ptr(ell), ptr(alpha), alpha.stride(0), ptr(g_mean), ptr(g_var), ldg,
+                              ptr(beta), ldb, sb, ptr(g_x), d, ptr(ws), n, ns, d, dp, q, stream()),
+        "cross_grad",
+    )
+    return g_x
+
+
+@_on_device
 def syrk(A, C, alpha=1.0, beta=0.0, cfg=None):
     """lower(C[b]) = alpha A[b]^T A[b] + beta C[b] for A [batch, k, >=n], C [batch, n, ld] (n, k multiples of 128)."""
     b, n, _ = C.shape

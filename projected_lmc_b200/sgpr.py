@@ -128,8 +128,10 @@ def prediction_state(engine, X, TY, U, comps, noise, max_tries=None):
     return dict(Luu=Luu, LB=LB, w=w, kss=kss, U=U, comps=comps)
 
 
-def predict_latents(engine, st, X, Xs, tile=65536):
-    """Latent posterior means / variances at Xs under the eval-mode SGPR covariance: ([q, n*], [q, n*])."""
+def predict_latents(engine, st, X, Xs, tile=65536, test_rows=False):
+    """Latent posterior means / variances at Xs under the eval-mode SGPR covariance: ([q, n*], [q, n*]).
+    ``test_rows``: the cross block is built with the test points as the rows of CrossGram (and transposed), so that
+    torch autograd reaches Xs through the block's adjoint."""
     q = st["kss"].shape[0]
     ns = Xs.shape[0]
     mean = torch.empty((q, ns), dtype=torch.float64, device=Xs.device)
@@ -143,7 +145,10 @@ def predict_latents(engine, st, X, Xs, tile=65536):
             _, xm = engine._sub_inputs(X, dims)
             full = len(dims) == U.shape[1] and tuple(dims) == tuple(range(U.shape[1]))
             Ug, xg = (U, xs) if full else (U[:, list(dims)], xs[:, list(dims)].contiguous())
-            b = CrossGram.apply(Ug, xg, xm, kid, ell, os_, False, ops.shape_of(c))
+            if test_rows:
+                b = CrossGram.apply(xg, Ug, xm, kid, ell, os_, False, ops.shape_of(c)).transpose(1, 2)
+            else:
+                b = CrossGram.apply(Ug, xg, xm, kid, ell, os_, False, ops.shape_of(c))
             Kus = b if Kus is None else Kus + b
         As = torch.linalg.solve_triangular(st["Luu"], Kus, upper=False)                      # [q, m, t]
         mean[:, s0:s0 + tile] = (As * st["w"]).sum(1)
